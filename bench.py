@@ -9,6 +9,7 @@ orientations of the figure-2 '2p0x_lr' rescan PSF (107^2), fp32.
 
   python bench.py [--gpus N] [--steps K] [--warmup W]       this repo (CUDA)
   python bench.py --impl reference ...                      CPU reference arm
+  python bench.py ... --dump-outputs DIR                    + the last timed frame as .npy
 
 With N > 1 (torchrun) every rank simulates and deconvolves its own frames
 (independent frames = the reference's own unit of parallel work: figure 2
@@ -22,19 +23,31 @@ Prints ONE JSON line on rank 0.
 `e2e` goes through the reference-facing API: line_sted_tools.Deconvolver --
 create_data_from_object(host object) + 64 x iterate() + read of `.estimate`.
 The reference arm runs the UNMODIFIED reference module from baseline/_ref/
-(a git-ignored copy made by __graft_entry__.build(); `kind: "reference"`),
-or the oracle port when that copy is absent (`kind: "port"`).
+(a git-ignored copy of the reference's figure_generation directory, where one
+was placed; `kind: "reference"`), or the oracle port when that copy is absent
+(`kind: "port"`).
+
+--dump-outputs DIR writes what the timed frame hands its caller, from the last
+timed step: DIR/estimate.npy (1, N, N) and DIR/noisy_measurement.npy /
+DIR/noiseless_measurement.npy (K, N, N), in the engine's precision (float32 or
+float64).  The files take at most 64 MB: an array too large for its share (half
+for the estimate, a quarter for each measurement) is replaced by the same fixed,
+seeded sample of pixels of every plane (K, P); at the defaults that is the two
+measurements.  Inputs and seeds depend only on the arguments, so two
+builds can be compared output for output.  Nothing is written to the tree.
 """
 import argparse
 import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True      # the tree may be read-only; leave it as it is
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -61,6 +74,8 @@ def parse_args():
                     help='N>1: independent frames per GPU (weak scaling, no collective) or the '
                          'K orientations of every frame split over the GPUs (strong scaling, one '
                          'NCCL all-reduce per RL iteration)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the outputs of the last timed step to DIR/<name>.npy (rank 0)')
     return ap.parse_args()
 
 
@@ -328,6 +343,29 @@ def ncu_facts(precision, N, K):
     return None
 
 
+DUMP_BYTES = 63 * 10 ** 6          # array data of --dump-outputs: 64 MB with room for the headers
+
+
+def dump_outputs(h, out_dir, dtype):
+    """What one frame hands its caller: the estimate (up to half of DUMP_BYTES whole) and the K
+    noisy / noiseless measurements (a quarter each).  An array that does not fit its share is
+    stored as the same seeded sample of pixel positions of every plane.  `dtype` is the
+    engine's precision, so nothing is rounded on the way out."""
+    from rescan_line_sted_b200 import _lib
+    os.makedirs(out_dir, exist_ok=True)
+    n = h.Ny * h.Nx
+    item = np.dtype(dtype).itemsize
+    for name, which, planes, share in (('estimate', _lib.ESTIMATE, 1, DUMP_BYTES // 2),
+                                       ('noisy_measurement', _lib.NOISY, h.K, DUMP_BYTES // 4),
+                                       ('noiseless_measurement', _lib.NOISELESS, h.K, DUMP_BYTES // 4)):
+        if planes * n * item <= share:
+            out = np.stack([h.get(which, k)[0] for k in range(planes)]).astype(dtype)
+        else:
+            pixels = np.sort(np.random.default_rng(0).choice(n, share // (planes * item), replace=False))
+            out = np.stack([h.get(which, k).reshape(-1)[pixels] for k in range(planes)]).astype(dtype)
+        np.save(os.path.join(out_dir, name + '.npy'), out)
+
+
 def time_frames(h, frame, seeds, barrier):
     barrier()
     h.timer_start()
@@ -416,6 +454,8 @@ def main():
     t_begin = time.perf_counter()
     ms_total = time_frames(h, frame_resident, [s + 1 + seed0 for s in range(args.steps)], barrier)
     sampler.window(t_begin, time.perf_counter())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(h, args.dump_outputs, np.float32 if args.precision == 'fp32' else np.float64)
     # Same K steps again with a CUDA-event pair around every launch (costs a few
     # microseconds of stream time per launch, so it is kept out of `value`): the
     # per-kernel durations behind `roofline` and `kernels`.
@@ -443,7 +483,7 @@ def main():
             return pinned_out
         api = 'DeconvHandle of the orientation-sharded deconvolver (upload_object, simulate, iterate, get)'
     else:
-        d = st.Deconvolver(psfs, output_prefix=os.path.join('/tmp', 'lsted_bench_%d_' % rank),
+        d = st.Deconvolver(psfs, output_prefix=os.path.join(tempfile.gettempdir(), 'lsted_bench_%d_' % rank),
                            verbose=False)
         d._handle, d._shape = h, (1, N, N)          # share the bench handle (OTFs already built)
         d._psf_key = tuple(id(p) for p in d.psfs)

@@ -1,20 +1,16 @@
-"""Import the UNMODIFIED reference module from /root/reference (build
-container) or from its git-ignored copy baseline/_ref/ that __graft_entry__.build()
-makes and gpurun ships to the GPU box.  Used by the golden-vector generator
-and by the CPU tests that pin the oracle.  matplotlib is not installed in the
-image and the reference imports (but never uses) it, so a stub is injected."""
+"""Import the UNMODIFIED reference module from a copy of the reference's
+figure_generation directory: $LSTED_REFERENCE_DIR, else the git-ignored
+baseline/_ref/.  Used by the golden-vector generators in tests/golden/; the
+test suite itself reads only the stored vectors.  The reference imports (but
+never uses) matplotlib, which need not be installed, so a stub is injected."""
 import importlib.util
 import os
 import sys
 import types
 import warnings
 
-_CANDIDATES = ('/root/reference/figure_generation',
-               os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))),
-                            'baseline', '_ref'))
-REFERENCE_DIR = os.environ.get('LSTED_REFERENCE_DIR') or next(
-    (d for d in _CANDIDATES if os.path.isfile(os.path.join(d, 'line_sted_tools.py'))),
-    _CANDIDATES[0])
+REFERENCE_DIR = os.environ.get('LSTED_REFERENCE_DIR') or os.path.join(
+    os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 'baseline', '_ref')
 
 
 def reference_available():

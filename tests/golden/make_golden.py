@@ -1,8 +1,7 @@
 #!/usr/bin/env python3
 """Generate the golden fixtures in this directory by running the UNMODIFIED
-reference (`/root/reference/figure_generation/line_sted_tools.py`).
-
-Run in the build container (the reference is not present on the GPU box):
+reference (`figure_generation/line_sted_tools.py`), read from
+$LSTED_REFERENCE_DIR or baseline/_ref/ (tests/_reference_loader.py):
     python tests/golden/make_golden.py
 Outputs (committed):
     psf_reports.npz      psf_report() dicts for four operating points

@@ -1,9 +1,8 @@
 #!/usr/bin/env python3
 """Golden vectors for the figure-3 scan-position engine (SURVEY.md 8f row 2), captured from the
 UNMODIFIED reference function `simulate_imaging`
-(/root/reference/figure_generation/line_sted_figure_3.py:76-273).
-
-Run in the build container (the reference is not on the GPU box):
+(figure_generation/line_sted_figure_3.py:76-273), read from $LSTED_REFERENCE_DIR or
+baseline/_ref/ (tests/_reference_loader.py):
     python tests/golden/make_golden_fig3.py
 The reference script calls main() at import and draws with matplotlib, so it is executed from
 its source text with that last call left out and with `generate_figure` / `animate` replaced by
@@ -13,7 +12,11 @@ recorders -- the simulation code itself runs untouched.  Output (committed): fig
    script's own size), as float64 arrays,
  * sum and max of every array of EVERY drawn frame (so all positions are pinned),
  * the call counts (scan positions, camera exposures) the appendix table publishes
-   (appendix.html:325-369).
+   (appendix.html:325-369);
+and fig3_object_lines.npz: `object_u8`, the 8-bit test_object_lines.tif every case crops.
+The committed copy of that image was read back from the stored frames (glow / excitation of
+the rot-0 frames is the object times a constant; the 89-valued background filled the pixels
+no stored excitation reaches) and reproduces every stored frame bit for bit.
 """
 import json
 import os
@@ -81,9 +84,12 @@ CASES = {
 }
 
 
+def lines_u8():
+    return sys.modules['np_tif'].tif_to_array(os.path.join(REFERENCE_DIR, 'test_object_lines.tif'))
+
+
 def make_object(ns, crop):
-    np_tif = sys.modules['np_tif']
-    obj = np_tif.tif_to_array(os.path.join(REFERENCE_DIR, 'test_object_lines.tif')) / 255 + 1e-6
+    obj = lines_u8() / 255 + 1e-6
     lo = (128 - crop) // 2
     return np.ascontiguousarray(obj[:, lo:lo + crop, lo:lo + crop])
 
@@ -115,6 +121,7 @@ def main():
         print(name, len(calls), 'frames')
     # the reference's own table (appendix.html:325-369): scan positions per method
     np.savez_compressed(os.path.join(HERE, 'fig3_frames.npz'), **store)
+    np.savez_compressed(os.path.join(HERE, 'fig3_object_lines.npz'), object_u8=lines_u8())
     with open(os.path.join(HERE, 'fig3_frames.json'), 'w') as f:
         json.dump(meta, f, indent=0)
 

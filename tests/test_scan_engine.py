@@ -28,16 +28,13 @@ def golden(golden_dir):
 
 
 def lines_object(crop, tile=1):
-    """test_object_lines.tif / 255 + 1e-6 like line_sted_figure_3.py:42, centre crop."""
-    from rescan_line_sted_b200 import np_tif
+    """test_object_lines.tif / 255 + 1e-6 like line_sted_figure_3.py:42, centre crop.  The 8-bit
+    128^2 image the golden frames were captured on is stored in tests/golden/fig3_object_lines.npz."""
     here = os.path.dirname(os.path.abspath(__file__))
-    for d in ('/root/reference/figure_generation', os.path.join(here, os.pardir, 'baseline', '_ref')):
-        path = os.path.join(d, 'test_object_lines.tif')
-        if os.path.isfile(path):
-            obj = np_tif.tif_to_array(path) / 255 + 1e-6
-            lo = (128 - crop) // 2
-            return np.tile(np.ascontiguousarray(obj[:, lo:lo + crop, lo:lo + crop]), (1, tile, tile))
-    pytest.skip('test_object_lines.tif not available (run __graft_entry__.build() in the build container)')
+    u8 = np.load(os.path.join(here, 'golden', 'fig3_object_lines.npz'))['object_u8']
+    obj = u8 / 255 + 1e-6
+    lo = (128 - crop) // 2
+    return np.tile(np.ascontiguousarray(obj[:, lo:lo + crop, lo:lo + crop]), (1, tile, tile))
 
 
 def run_case(sim, meta):
