@@ -65,6 +65,7 @@ def test_tensor_map_row_staging_is_bit_identical(shape, K):
     est = {}
     for tma in (0, 1, 2):   # 2: also the two-buffer ROW_MID (measurement rows read in place)
         h = _lib.DeconvHandle(lib, psfs, shape, precision=32)
+        assert h.info().Lx == 2160          # the rows run the 2160 plan, where row_tma applies
         h.set_option('row_tma', tma)
         h.create_data(x, 1e6 * x.size, 1)
         h.iterate(3)
@@ -76,7 +77,7 @@ def test_tensor_map_row_staging_is_bit_identical(shape, K):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize('shape,K', [((2048, 64), 2), ((2048, 2048), 3), ((2001, 1030), 2)])
+@pytest.mark.parametrize('shape,K', [((2048, 64), 2), ((2048, 2048), 3), ((2101, 1030), 2)])
 def test_sub_block_column_ctas_are_bit_identical(shape, K):
     """Column kernels on centred real OTFs as sub-block CTAs (2 of 4 columns, two CTAs per
     SM; option `col_sub`, default on) against the whole-block CTAs: bit-identical estimates."""
@@ -90,6 +91,7 @@ def test_sub_block_column_ctas_are_bit_identical(shape, K):
     est = {}
     for sub in (0, 1):
         h = _lib.DeconvHandle(lib, psfs, shape, precision=32)
+        assert h.info().Ly == 2160          # the columns run the 2160 plan, where col_sub applies
         h.set_option('col_sub', sub)
         h.create_data(x, 1e6 * x.size, 1)
         h.iterate(3)

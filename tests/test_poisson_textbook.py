@@ -8,62 +8,12 @@ import ctypes
 
 import numpy as np
 import pytest
-from scipy.special import gammaln
 
 import emul_support
+from _poisson_replay import (assert_field, replay_counts, replay_field, textbook_multiplication,
+                             textbook_ptrs)
 
 dp = ctypes.POINTER(ctypes.c_double)
-M32 = np.uint64(0xFFFFFFFF)
-
-
-def philox4x32_10(c0, c1, c2, c3, k0, k1):
-    c0, c1, c2, c3 = (np.asarray(c, dtype=np.uint64) for c in (c0, c1, c2, c3))
-    k0, k1 = np.uint64(k0), np.uint64(k1)
-    for _ in range(10):
-        p0 = np.uint64(0xD2511F53) * c0
-        p1 = np.uint64(0xCD9E8D57) * c2
-        hi0, lo0, hi1, lo1 = p0 >> np.uint64(32), p0 & M32, p1 >> np.uint64(32), p1 & M32
-        c0, c1, c2, c3 = hi1 ^ c1 ^ k0, lo1, hi0 ^ c3 ^ k1, lo0
-        k0 = (k0 + np.uint64(0x9E3779B9)) & M32
-        k1 = (k1 + np.uint64(0xBB67AE85)) & M32
-    return c0, c1, c2, c3
-
-
-def u01(hi, lo):
-    return (((hi << np.uint64(32)) | lo) >> np.uint64(11)).astype(np.float64) * 2.0 ** -53
-
-
-def textbook_ptrs(lam, seed, pixels):
-    """numpy's legacy `random_poisson_ptrs`, attempt `att` drawn from counter
-    (pixel lo, pixel hi, image 0, att) with key = seed."""
-    slam, loglam = np.sqrt(lam), np.log(lam)
-    b = 0.931 + 2.53 * slam
-    a = -0.059 + 0.02483 * b
-    invalpha = 1.1239 + 1.1328 / (b - 3.4)
-    vr = 0.9277 - 3.6224 / (b - 2.0)
-    out = np.full(pixels.shape, -1.0)
-    todo = np.arange(pixels.size)
-    for att in range(64):
-        if todo.size == 0:
-            break
-        p = pixels[todo].astype(np.uint64)
-        zero = np.zeros_like(p)
-        v = philox4x32_10(p & M32, p >> np.uint64(32), zero, zero + np.uint64(att),
-                          seed & 0xFFFFFFFF, seed >> 32)
-        U = u01(v[0], v[1]) - 0.5
-        V = u01(v[2], v[3])
-        us = 0.5 - np.abs(U)
-        with np.errstate(divide='ignore', invalid='ignore'):
-            k = np.floor((2.0 * a / us + b) * U + lam + 0.43)
-            squeeze = (us >= 0.07) & (V <= vr)
-            skip = (k < 0.0) | ((us < 0.013) & (V > us))
-            exact = (np.log(V) + np.log(invalpha) - np.log(a / (us * us) + b)
-                     <= -lam + k * loglam - gammaln(k + 1.0))
-        accept = squeeze | (~skip & exact)
-        out[todo[accept]] = k[accept]
-        todo = todo[~accept]
-    assert todo.size == 0
-    return out
 
 
 @pytest.mark.parametrize('lam', [10.0, 12.5, 17.0, 30.0, 100.0, 1e4, 1.8e7])
@@ -80,35 +30,6 @@ def test_sampler_is_textbook_ptrs_on_the_same_counters(lam):
     assert np.array_equal(got, want)
 
 
-def textbook_multiplication(lam, seed, pixels):
-    """Knuth's multiplication method (numpy's legacy `random_poisson_mult`): count uniforms
-    until their product drops to exp(-lam); each Philox call supplies two of them."""
-    enlam = np.exp(-lam)
-    out = np.zeros(pixels.size)
-    prod = np.ones(pixels.size)
-    running = np.ones(pixels.size, dtype=bool)
-    for att in range(200):
-        idx = np.flatnonzero(running)
-        if idx.size == 0:
-            break
-        p = pixels[idx].astype(np.uint64)
-        zero = np.zeros_like(p)
-        v = philox4x32_10(p & M32, p >> np.uint64(32), zero, zero + np.uint64(att),
-                          seed & 0xFFFFFFFF, seed >> 32)
-        ua, ub = u01(v[0], v[1]), u01(v[2], v[3])
-        prod[idx] *= ua
-        done = ~(prod[idx] > enlam)
-        running[idx[done]] = False
-        idx, ub = idx[~done], ub[~done]     # the second uniform: pixels still running only
-        out[idx] += 1.0
-        prod[idx] *= ub
-        done = ~(prod[idx] > enlam)
-        running[idx[done]] = False
-        out[idx[~done]] += 1.0
-    assert not running.any()
-    return out
-
-
 @pytest.mark.parametrize('lam', [0.5, 5.0, 9.9])
 def test_small_lambda_sampler_is_the_multiplication_method(lam):
     lib = emul_support.emulator_library()
@@ -119,3 +40,52 @@ def test_small_lambda_sampler_is_the_multiplication_method(lam):
     lib.cdll.emul_poisson(lam, seed, first, n, got.ctypes.data_as(dp))
     want = textbook_multiplication(lam, seed, first + np.arange(n, dtype=np.int64))
     assert np.array_equal(got, want)
+
+
+def test_field_check_has_teeth():
+    """The whole-field comparison the GPU tests make (tests/_poisson_replay.py) fails on one
+    pixel off by one count and on a field drawn for another image index."""
+    rng = np.random.default_rng(4)
+    lam = np.concatenate([np.zeros(300), rng.uniform(0.0, 10.0, 1500), rng.uniform(10.0, 1e4, 1500),
+                          rng.uniform(1.9e7, 2.1e7, 300)]).reshape(1, 36, 100)
+    seed = 0xC0FFEE
+    field = replay_field(lam, seed, 1, np.float32)
+    assert_field(field, lam, seed, 1, np.float32)
+    for i in (np.flatnonzero(lam == 0)[7], np.flatnonzero((lam > 0) & (lam < 10))[11],
+              np.flatnonzero((lam >= 10) & (lam < 1e4))[13]):
+        bad = field.copy()
+        bad.flat[i] += 1.0
+        with pytest.raises(AssertionError, match='pixel %d ' % i):
+            assert_field(bad, lam, seed, 1, np.float32)
+    with pytest.raises(AssertionError, match='pixels differ'):
+        assert_field(field, lam, seed, 0, np.float32)
+    # above 2^24 the fp32 field holds even counts only: the replay rounds the same way
+    big = field[lam > 2 ** 24]
+    assert (big % 2 == 0).all() and not (replay_counts(lam, seed, 1)[lam > 2 ** 24] % 2 == 0).all()
+
+
+@pytest.mark.parametrize('fast', [1, 0])
+@pytest.mark.parametrize('precision', [32, 64])
+def test_cpu_replay_noise_field_is_the_textbook_field(precision, fast):
+    """create_data's noise field on the CPU replay of the kernels (fast 2160 rows and generic
+    rows, both images) is replay_field of its noiseless images, pixel for pixel."""
+    from rescan_line_sted_b200 import _lib
+    lib = emul_support.emulator_library()
+    rng = np.random.default_rng(6)
+    ny, nx, seed = 4, 2048, 0x5EED
+    psfs = rng.random((2, 3, 9))
+    psfs /= psfs.sum(axis=(1, 2), keepdims=True)
+    obj = rng.random((1, ny, nx)) * 8.0
+    obj[0, :, 100:400] = 0.0            # dark: exact zeros
+    obj[0, :, 700:1200] *= 1e3          # PTRS
+    obj[0, :, 1500:1600] = 2e7          # fp32 rounds the counts
+    h = _lib.DeconvHandle(lib, psfs, (ny, nx), precision=precision)
+    h.set_option('fast_path', fast)
+    h.create_data(obj, None, seed)
+    assert h.info().Lx == 2160
+    dtype = np.float32 if precision == 32 else np.float64
+    for k in range(2):
+        lam = h.get(_lib.NOISELESS, k)
+        assert (lam == 0).any() and ((lam > 0) & (lam < 10)).any() and (lam > 2 ** 24).any()
+        assert_field(h.get(_lib.NOISY, k), lam, seed, k, dtype)
+    h.close()
