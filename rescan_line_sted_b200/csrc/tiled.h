@@ -69,11 +69,12 @@ template <typename T, class BK> class TiledEngine : public EngineBase {
         win2 = (T*)bk.alloc(sizeof(T) * wpix);
         winK = (T*)bk.alloc(sizeof(T) * wpix * K);
         stage64 = (double*)bk.alloc(sizeof(double) * npix);
+        object64 = (double*)bk.alloc(sizeof(double) * npix);
         partial = (double*)bk.alloc(sizeof(double) * 1024);
     }
     ~TiledEngine() {
         void* all[] = {true_object, estimate, norm, noiseless, noisy, ratio, win1, win2, winK,
-                       stage64, partial, halo_send, halo_recv, stage_region,
+                       stage64, object64, partial, halo_send, halo_recv, stage_region,
                        ft_scratch, tw_dx, tw_dy, spec_direct};
         for (size_t i = 0; i < sizeof(all) / sizeof(all[0]); ++i) bk.free(all[i]);
     }
@@ -230,11 +231,14 @@ template <typename T, class BK> class TiledEngine : public EngineBase {
         }
     }
 
-    void upload_object(const double* obj_host) { bk.upload(stage64, obj_host, sizeof(double) * npix); }
+    // The staged object has a buffer of its own: stage64 is the host-transfer scratch of every
+    // get / set / H / H_t / ft_error, any of which may run between upload_object and simulate
+    // (a frame loop uploads once and simulates a new noise field per frame).
+    void upload_object(const double* obj_host) { bk.upload(object64, obj_host, sizeof(double) * npix); }
     void simulate(double total_brightness, bool rescale, unsigned long long seed) {
         double s = 1.0;
-        if (rescale) s = total_brightness / bk.sum(stage64, npix, partial);
-        bk.cast_in(true_object, stage64, npix, s);
+        if (rescale) s = total_brightness / bk.sum(object64, npix, partial);
+        bk.cast_in(true_object, object64, npix, s);
         for (int ty = ty0; ty < ty1; ++ty)
             for (int tx = tx0; tx < tx1; ++tx) {
                 window(WIN_LOAD, ty, tx, win1, true_object, 0, 1, false);
@@ -403,7 +407,7 @@ template <typename T, class BK> class TiledEngine : public EngineBase {
     std::vector<Rect> send_rect, recv_rect;
     T *true_object, *estimate, *norm, *noiseless, *noisy, *ratio, *win1, *win2, *winK;
     T *halo_send, *halo_recv;
-    double *stage64, *partial, *stage_region;
+    double *stage64, *object64, *partial, *stage_region;
     T* ft_scratch = 0;                                      // ft_error (lazy)
     cplx<double>*tw_dx = 0, *tw_dy = 0, *spec_direct = 0;
 

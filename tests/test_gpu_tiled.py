@@ -1,7 +1,8 @@
-"""Tiled engine on the GPU with the 2160 fast-path tiles: against the oracle at a
-two-tile size, and at config-5 scale (8192^2 tiles, fp64) through exact local
-checks: a linear convolution is local, so any patch of the tiled result must
-equal the oracle's convolution of the patch plus its halo."""
+"""Tiled engine on the GPU at config-5 scale (8192^2 tiles, fp64) through exact
+local checks: a linear convolution is local, so any patch of the tiled result
+must equal the oracle's convolution of the patch plus its halo.  The tile grids,
+PSF shapes and window lengths against the whole-image oracle are in
+test_gpu_tiled_parity.py."""
 import numpy as np
 import pytest
 
@@ -12,27 +13,6 @@ pytestmark = pytest.mark.gpu
 
 def rel_l2(a, b):
     return np.linalg.norm(np.ravel(a) - np.ravel(b)) / np.linalg.norm(np.ravel(b))
-
-
-@pytest.mark.parametrize('precision,tol', [(64, 1e-12), (32, 1e-5)])
-def test_two_tiles_against_oracle(precision, tol):
-    from rescan_line_sted_b200 import _lib
-    rng = np.random.default_rng(1)
-    psfs = rng.random((2, 9, 11))
-    shape = (2200, 2300)                      # does not fit one 2160 window -> 2 x 2 tiles
-    x = rng.random((1,) + shape)
-    h = _lib.DeconvHandle(_lib.get(), psfs, shape, precision=precision, tile_fft_len=2160)
-    info = h.info()
-    assert (info.tiles_y, info.tiles_x) == (2, 2) and info.Lx == 2160
-    o = orc.Deconvolver([p[None] for p in psfs])
-    assert rel_l2(h.H(x), np.concatenate(o.H(x))) < tol
-    h.create_data(x, 1e9, 3)
-    o.create_data_from_object(x, 1e9, 3)
-    o.noisy_measurement = [h.get(_lib.NOISY, k) for k in range(2)]
-    h.iterate(2)
-    o.iterate(), o.iterate()
-    assert rel_l2(h.get(_lib.ESTIMATE), o.estimate) < 10 * tol
-    h.close()
 
 
 def test_config5_scale_local_exactness():
