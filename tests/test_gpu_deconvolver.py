@@ -8,6 +8,7 @@ import os
 import numpy as np
 import pytest
 
+from _local_error import check_local, local_errors
 from oracle import line_sted_oracle as orc
 
 pytestmark = pytest.mark.gpu
@@ -68,11 +69,17 @@ def test_H_and_Ht_ragged_shapes(st, precision, shape, pshape, tmp_path):
     d = st.Deconvolver(psfs, output_prefix=str(tmp_path) + '/h_', verbose=False)
     o = orc.Deconvolver(psfs)
     x = rng.random(shape)
-    for a, b in zip(d.H(x), o.H(x)):
+    got, want = d.H(x), o.H(x)
+    for a, b in zip(got, want):
         assert a.shape == b.shape
         assert rel_l2(a, b) < tol
     y = [rng.random(shape) for _ in psfs]
-    assert rel_l2(d.H_t(y, normalize=False), o.H_t(y, normalize=False)) < tol
+    Ht, Ht_want = d.H_t(y, normalize=False), o.H_t(y, normalize=False)
+    assert rel_l2(Ht, Ht_want) < tol
+    info, bits = d._handle.info(), int(precision[2:])
+    label = 'ragged %s psf %s' % (shape[1:], pshape[1:])
+    check_local([(label + ' H', local_errors(np.concatenate(got), np.concatenate(want), info, bits)),
+                 (label + ' Ht', local_errors(Ht, Ht_want, info, bits))])
     assert rel_l2(d.H_t(y), o.H_t(y)) < tol
     assert rel_l2(d.H_t_normalization, o.H_t_normalization) < tol
 

@@ -20,6 +20,7 @@ import numpy as np
 import pytest
 
 import bench
+from _local_error import check_local, local_errors
 from _poisson_replay import assert_field
 from oracle import line_sted_oracle as orc
 
@@ -152,21 +153,30 @@ def check_against_oracle(h, c, label):
     from rescan_line_sted_b200 import _lib
     x, y, B, Hx, Hty, noiseless, noisy, est = oracle_results(c.shape, c.psf, c.K, c.obj)
     tol_op, tol_it = TOL[c.precision]
-    err = {'H': rel_l2(h.H(x), Hx), 'Ht': rel_l2(h.Ht(y, False), Hty)}
+    info = h.info()
+    got = {'H': h.H(x), 'Ht': h.Ht(y, False)}
     h.create_data(x, B, 3)
-    err['noiseless'] = max(rel_l2(h.get(_lib.NOISELESS, k), noiseless[k]) for k in range(c.K))
+    got['noiseless'] = np.concatenate([h.get(_lib.NOISELESS, k) for k in range(c.K)])
     for k in range(c.K):
         h.set(_lib.NOISY, k, noisy[k])
     for n in (1, 2):
         h.iterate(1)
-        got = h.get(_lib.ESTIMATE)
-        assert np.isfinite(got).all()
-        err['iter%d' % n] = rel_l2(got, est[n - 1])
+        got['iter%d' % n] = h.get(_lib.ESTIMATE)
+        assert np.isfinite(got['iter%d' % n]).all()
+    want = {'H': Hx, 'Ht': Hty, 'noiseless': np.concatenate(noiseless),
+            'iter1': est[0], 'iter2': est[1]}
+    err = {'H': rel_l2(got['H'], Hx), 'Ht': rel_l2(got['Ht'], Hty),
+           'noiseless': max(rel_l2(got['noiseless'][k], noiseless[k]) for k in range(c.K)),
+           'iter1': rel_l2(got['iter1'], est[0]), 'iter2': rel_l2(got['iter2'], est[1])}
     print('measured %s (fp%d): %s' % (label, c.precision,
                                       ', '.join('%s %.2e' % kv for kv in err.items())))
+    local = [('%s %s' % (label, name), local_errors(got[name], want[name], info, c.precision,
+                                                   estimate=name.startswith('iter')))
+             for name in want]
+    check_local(local)
     for name, e in err.items():
         assert e < (tol_it if name.startswith('iter') else tol_op), (label, name, e)
-    return got
+    return got['iter2']
 
 
 @pytest.mark.parametrize('name', sorted(CASES))

@@ -3,6 +3,7 @@ and the oracle at a size the oracle finishes in seconds."""
 import numpy as np
 import pytest
 
+from _local_error import check_local, local_errors
 from oracle import line_sted_oracle as orc
 
 pytestmark = pytest.mark.gpu
@@ -28,19 +29,29 @@ def test_fast_path_matches_oracle_and_generic(precision, tol, shape):
     h = _lib.DeconvHandle(lib, psfs, shape, precision=precision)
     info = h.info()
     assert (info.Ly, info.Lx) == (2160, 2160)
-    assert rel_l2(h.H(x), Hx) < tol
-    assert rel_l2(h.Ht(y, False), Hty) < tol
+    H, Ht = h.H(x), h.Ht(y, False)
+    assert rel_l2(H, Hx) < tol
+    assert rel_l2(Ht, Hty) < tol
     h.create_data(x, 1e9, 0)
     noisy = [h.get(_lib.NOISY, k) for k in range(2)]
     h.iterate(2)
     o.create_data_from_object(x, 1e9, 0)
     o.noisy_measurement = noisy
     o.iterate(), o.iterate()
-    assert rel_l2(h.get(_lib.ESTIMATE), o.estimate) < 10 * tol
+    est = h.get(_lib.ESTIMATE)
+    assert rel_l2(est, o.estimate) < 10 * tol
+    label = 'fast path %dx%d' % shape
+    check_local([(label + ' H', local_errors(H, Hx, info, precision)),
+                 (label + ' Ht', local_errors(Ht, Hty, info, precision)),
+                 (label + ' noiseless', local_errors(np.concatenate([h.get(_lib.NOISELESS, k) for k in range(2)]),
+                                                     np.concatenate(o.noiseless_measurement), info, precision)),
+                 (label + ' iter2', local_errors(est, o.estimate, info, precision, estimate=True))])
     if precision == 32:   # the generic kernels fit in shared memory for fp32 only
         g = _lib.DeconvHandle(lib, psfs, shape, precision=precision)
         g.set_option('fast_path', 0)
-        assert rel_l2(g.H(x), Hx) < tol
+        gH = g.H(x)
+        assert rel_l2(gH, Hx) < tol
+        check_local([(label + ' generic H', local_errors(gH, Hx, info, precision))])
         g.create_data(x, 1e9, 0)
         for k in range(2):
             g.set(_lib.NOISY, k, noisy[k])

@@ -9,6 +9,7 @@ import numpy as np
 import pytest
 
 import bench
+from _local_error import check_local, local_errors
 from oracle import line_sted_oracle as orc
 
 pytestmark = pytest.mark.gpu
@@ -162,12 +163,12 @@ def test_forward_model_against_oracle_on_all_orientations(setup):
     obj = bench.synthetic_object(N)
     h.create_data(obj, bench.total_brightness(N), 0)
     scaled = obj * (bench.total_brightness(N) / obj.sum())
-    worst = 0.0
     with scipy.fft.set_workers(os.cpu_count()):
-        for k in range(K):
-            want = np.clip(orc.fftconvolve_same(scaled, psfs[k]), 0, None)
-            worst = max(worst, rel_l2(h.get(_lib.NOISELESS, k), want))
+        want = np.concatenate([np.clip(orc.fftconvolve_same(scaled, psfs[k]), 0, None) for k in range(K)])
+    got = np.concatenate([h.get(_lib.NOISELESS, k) for k in range(K)])
+    worst = max(rel_l2(got[k], want[k]) for k in range(K))
     _record('forward_O1_all16_fp32', worst)
+    check_local([('forward O1 noiseless', local_errors(got, want, h.info(), 32))])
     assert worst < TOL
 
 
@@ -184,8 +185,11 @@ def test_objects_O2_O3_create_inject_iterate_both_clip_orders(setup, name):
         o.create_data_from_object(obj, total_brightness=B, random_seed=0)
         h.set_option('exact_clip', 0)
         h.create_data(obj, B, 0)
-        worst = max(rel_l2(h.get(_lib.NOISELESS, k), o.noiseless_measurement[k]) for k in range(K))
+        got = np.concatenate([h.get(_lib.NOISELESS, k) for k in range(K)])
+        worst = max(rel_l2(got[k], o.noiseless_measurement[k]) for k in range(K))
         _record('forward_%s_fp32' % name, worst)
+        check_local([('forward %s noiseless' % name,
+                      local_errors(got, np.concatenate(o.noiseless_measurement), h.info(), 32))])
         assert worst < TOL
         est = {}
         for n_it in (1, 2):
@@ -203,6 +207,8 @@ def test_objects_O2_O3_create_inject_iterate_both_clip_orders(setup, name):
             assert np.isfinite(got).all()
             err = rel_l2(got, est[n_it])
             _record('estimate_%s_iter%d_exact_clip%d_fp32' % (name, n_it, exact), err)
+            check_local([('%s iter%d exact_clip %d' % (name, n_it, exact),
+                          local_errors(got, est[n_it], h.info(), 32, estimate=True))])
             assert err < TOL_ITER[n_it], (name, exact, n_it, err)
     h.set_option('exact_clip', 0)
     h.set_option('forget_normalization', 1)

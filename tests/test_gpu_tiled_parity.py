@@ -19,6 +19,7 @@ import numpy as np
 import pytest
 
 import bench
+from _local_error import check_local, local_errors
 from oracle import line_sted_oracle as orc
 
 pytestmark = pytest.mark.gpu
@@ -186,14 +187,19 @@ def open_handle(c):
 def check_against_oracle(h, c, label):
     from rescan_line_sted_b200 import _lib
     r = oracle_results(c.shape, c.psf, c.K, c.obj)
-    mask = seam_mask(c.shape, h.info(), make_psfs(c.psf, c.K).shape[1:])
-    err = {'H': errors(h.H(r['x']), r['H'], mask),
-           'Ht': errors(h.Ht(r['y'], False), r['Ht'], mask),
+    info = h.info()
+    mask = seam_mask(c.shape, info, make_psfs(c.psf, c.K).shape[1:])
+    H, Ht = h.H(r['x']), h.Ht(r['y'], False)
+    err = {'H': errors(H, r['H'], mask),
+           'Ht': errors(Ht, r['Ht'], mask),
            'Ht_norm': errors(h.Ht(r['y'], True), r['Ht_norm'], mask),
            'norm': errors(h.get(_lib.NORMALIZATION), r['norm'], mask)}
+    local = [(label + ' H', local_errors(H, r['H'], info, c.precision)),
+             (label + ' Ht', local_errors(Ht, r['Ht'], info, c.precision))]
     h.create_data(r['x'], r['B'], 3)
-    err['noiseless'] = errors(np.concatenate([h.get(_lib.NOISELESS, k) for k in range(c.K)]),
-                              r['noiseless'], mask)
+    noiseless = np.concatenate([h.get(_lib.NOISELESS, k) for k in range(c.K)])
+    err['noiseless'] = errors(noiseless, r['noiseless'], mask)
+    local.append((label + ' noiseless', local_errors(noiseless, r['noiseless'], info, c.precision)))
     for k in range(c.K):
         h.set(_lib.NOISY, k, r['noisy'][k])
     for n in (1, 2):
@@ -201,9 +207,12 @@ def check_against_oracle(h, c, label):
         got = h.get(_lib.ESTIMATE)
         assert np.isfinite(got).all() and got.min() >= 0
         err['iter%d' % n] = errors(got, r['est'][n - 1], mask)
+        local.append(('%s iter%d' % (label, n),
+                      local_errors(got, r['est'][n - 1], info, c.precision, estimate=True)))
     assert h.info().iterations_done == 2
     print('measured %s (fp%d): %s' % (label, c.precision, ', '.join(
         '%s %.2e/%.2e' % (name, l2, seam) for name, (l2, seam) in err.items())))
+    check_local(local)
     tol_op, tol_it = TOL[c.precision]
     for name, (l2, seam) in err.items():
         tol = tol_it if name.startswith('iter') else tol_op
