@@ -14,7 +14,6 @@
 #include <string>
 #include <map>
 #include <vector>
-#include <type_traits>
 
 #include "../../include/lsted.h"
 #include "engine.h"
@@ -22,6 +21,7 @@
 #include "conv_fast.cuh"
 #include "ew_bodies.cuh"
 #include "psf_kernels.cuh"
+#include "dispatch.h"
 
 namespace lsted {
 struct ApiError { int code; std::string msg; };
@@ -60,7 +60,7 @@ struct DeviceCtx {
     }
 };
 
-// Compile-time plans of the fast path (conv_fast.cuh): 2160 = 16 * 9 * 15.
+// Launch bounds of the fast-path kernels (plans and selection: dispatch.h)
 #ifndef LSTED_ROW_LEAN_CTAS
 #define LSTED_ROW_LEAN_CTAS 6   // "lean" ROW_MID (two shared-memory buffers, 35 KB): CTAs per SM -> 64 registers, no spills
 #endif
@@ -70,27 +70,7 @@ struct DeviceCtx {
 #ifndef LSTED_ROW_RESIDENT_THREADS
 #define LSTED_ROW_RESIDENT_THREADS 480  // 3 row CTAs per SM: no register spills
 #endif
-#ifndef LSTED_FAST_C32
-#define LSTED_FAST_C32 4
-#endif
-#ifndef LSTED_FAST_CS32
-#define LSTED_FAST_CS32 2   // columns per sub-block column CTA (real OTFs): 2 CTAs per SM
-#endif
-#ifndef LSTED_FAST_PR
-#define LSTED_FAST_PR 1
-#endif
-typedef lsted::FastPlan<float, 16, 9, 15, 144, LSTED_FAST_C32, LSTED_FAST_PR, LSTED_FAST_CS32> Plan2160f;
-#ifndef LSTED_FP64_PR
-#define LSTED_FP64_PR 1   // row pairs per CTA of the fp64 plan (A/B at build time; 2: row_mid +13 %)
-#endif
-#ifndef LSTED_FP64_CS
-#define LSTED_FP64_CS 1   // columns per column CTA of the fp64 plan (1 of 2: sub-block CTAs; 2: col_h +15 %, col_ht +35 %)
-#endif
-typedef lsted::FastPlan<double, 16, 9, 15, 144, 2, LSTED_FP64_PR, LSTED_FP64_CS> Plan2160d;
-
 // G: image geometry known at compile time (the 2048-wide / 107-wide-PSF headline case) or not
-typedef lsted::RowGeomFixed<2048, 53> RowGeom2048;
-typedef lsted::RowGeomFixed<2048, 0> RowGeom2048c;    // centred real OTFs: no crop offset
 template <int MODE, class P, class G = lsted::RowGeomRuntime, int TMA = 0>
 __global__ void __launch_bounds__(P::ROW_THREADS, TMA == 2 ? (MODE == lsted::ROW_MID ? LSTED_ROW_LEAN_CTAS : 4) : sizeof(typename P::T) == 4 ? (MODE == lsted::ROW_INV_SIM ? LSTED_ROW_SIM_CTAS : LSTED_ROW_RESIDENT_THREADS / P::ROW_THREADS) : 1)
 row_fast_kernel(const __grid_constant__ lsted::RowArgs<typename P::T> a) {
@@ -105,7 +85,6 @@ row_fast_kernel(const __grid_constant__ lsted::RowArgs<typename P::T> a) {
 #ifndef LSTED_ROW2_CTAS
 #define LSTED_ROW2_CTAS 3
 #endif
-typedef lsted::FastPlan2<float, 48, 45, LSTED_FAST_C32, 2> Plan2160f2;
 template <int MODE, class P, class G = lsted::RowGeomRuntime>
 __global__ void __launch_bounds__(P::ROW_THREADS, LSTED_ROW2_CTAS)
 row2_fast_kernel(const __grid_constant__ lsted::RowArgs<typename P::T> a) {
@@ -126,8 +105,6 @@ row_mid_dual_kernel(const __grid_constant__ lsted::RowArgs<typename P::T> a) {
     lsted::row_mid_dual_body<P>(cx, blockIdx.x, a, smem_raw, &r);
 }
 
-typedef lsted::ColGeomFixed<2048, 53> ColGeom2048;
-typedef lsted::ColGeomFixed<2048, 0> ColGeom2048c;    // centred real OTFs: no crop offset
 // sub-block column CTAs (real OTFs): CS of the C columns of a block, two CTAs per SM
 template <int MODE, class P, class G = lsted::ColGeomRuntime>
 __global__ void __launch_bounds__(P::SUB_THREADS, 2)
@@ -370,18 +347,15 @@ static NcclApi& nccl_api() {
 // ---------------------------------------------------------------------------
 // CUDA backend of the engine
 // ---------------------------------------------------------------------------
-enum KernelKind { KK_ROW_FWD = 0, KK_ROW_INV_STORE, KK_ROW_INV_SIM, KK_ROW_MID, KK_ROW_FINAL,
-                  KK_COL_OTF, KK_COL_H, KK_COL_HT, KK_EW };
-
 // Deconvolver handles alive in this process: with many of them (figure 2 iterates 24 round-robin,
 // each on its own stream) the GPU is kept busy by the other handles' kernels and spreading one
 // frame's orientations over more CTAs only adds work (measured: 24 handles 6.5 -> 7.5 us / iteration).
 static int g_live_backends = 0;
 
-class CudaBackend {
+class CudaBackend : public lsted::KernelSelection {
   public:
     explicit CudaBackend(int device) : device_(device), stream_(0), bytes_(0), profile_(false),
-                                       use_fast_(true), t0_(0), t1_(0), num_sms_(148) {
+                                       t0_(0), t1_(0), num_sms_(148) {
         int count = 0;
         CUDA_CHECK(cudaGetDeviceCount(&count));
         if (device < 0 || device >= count) {
@@ -398,18 +372,6 @@ class CudaBackend {
         ++g_live_backends;
         memset(prof_ms_, 0, sizeof(prof_ms_));
         memset(prof_n_, 0, sizeof(prof_n_));
-        const char* dual = getenv("LSTED_ROW_DUAL");   // A/B switch, same as option "row_dual"
-        if (dual) row_dual_ = atoi(dual) != 0;
-        const char* plan2 = getenv("LSTED_ROW_PLAN2");  // A/B switch, same as option "row_plan2"
-        if (plan2) row_plan2_ = atoi(plan2) != 0;
-        const char* rt = getenv("LSTED_ROW_TMA");       // A/B switch: spectrum chunks by tensor-map copies
-        if (rt) row_tma_ = atoi(rt);   // 0 off, 1 tensor-map copies, 2 + "lean" ROW_MID
-        const char* cs = getenv("LSTED_COL_SUB");       // A/B switch, same as option "col_sub"
-        if (cs) col_sub_ = atoi(cs) != 0;
-        const char* ro = getenv("LSTED_REAL_OTF");      // A/B switch: centred real OTFs (read at set_psfs)
-        if (ro) real_otf_ = atoi(ro) != 0;
-        const char* pf = getenv("LSTED_PREFETCH");      // A/B switch, same as option "prefetch"
-        if (pf) prefetch_ = atoi(pf) != 0;
         const char* pq = getenv("LSTED_PREFETCH_CTAS_PER_SM");   // prefetch distance in CTAs per SM
         if (pq && atoi(pq) > 0) { prefetch_quarters_ = atoi(pq); prefetch_final_quarters_ = 0; }
     }
@@ -436,22 +398,22 @@ class CudaBackend {
         NCCL_CHECK(nccl_api().CommInitRank(&comm_, world, id, rank));
     }
     void all_reduce_sum(float* p, size_t n) {
-        before(KK_EW);
+        before(lsted::KK_EW);
         NCCL_CHECK(nccl_api().AllReduce(p, p, n, ncclFloat, ncclSum, comm_, stream_));
         after();
     }
     void all_reduce_sum(double* p, size_t n) {
-        before(KK_EW);
+        before(lsted::KK_EW);
         NCCL_CHECK(nccl_api().AllReduce(p, p, n, ncclDouble, ncclSum, comm_, stream_));
         after();
     }
     void broadcast(float* p, size_t n, int root) {
-        before(KK_EW);
+        before(lsted::KK_EW);
         NCCL_CHECK(nccl_api().Broadcast(p, p, n, ncclFloat, root, comm_, stream_));
         after();
     }
     void broadcast(double* p, size_t n, int root) {
-        before(KK_EW);
+        before(lsted::KK_EW);
         NCCL_CHECK(nccl_api().Broadcast(p, p, n, ncclDouble, root, comm_, stream_));
         after();
     }
@@ -598,7 +560,7 @@ class CudaBackend {
         }
         unsigned long long* mc_flags = (unsigned long long*)((char*)nvls_mcp_ + nvls_data_bytes_);
         const unsigned long long* uc_flags = (const unsigned long long*)((char*)nvls_uc_ + nvls_data_bytes_);
-        before(KK_EW);
+        before(lsted::KK_EW);
         // 32 CTAs x 512 threads: measured on 8 GPUs (17.8 MB): 0.061 ms, of which 0.024 ms are the two
         // cross-GPU barriers; 148 CTAs: 0.072, 8 CTAs: 0.065 (scripts/nvls_sweep.py)
         const int ctas = nvls_ctas_ > 0 && nvls_ctas_ <= num_sms_ ? nvls_ctas_ : (num_sms_ < 32 ? num_sms_ : 32);
@@ -616,7 +578,7 @@ class CudaBackend {
     template <typename T> void exchange(int npeers, const int* peers, T* const* send, const size_t* nsend,
                                         T* const* recv, const size_t* nrecv) {
         const ncclDataType_t dt = sizeof(T) == 4 ? ncclFloat : ncclDouble;
-        before(KK_EW);
+        before(lsted::KK_EW);
         NCCL_CHECK(nccl_api().GroupStart());
         for (int i = 0; i < npeers; ++i) {
             if (nsend[i]) NCCL_CHECK(nccl_api().Send(send[i], nsend[i], dt, peers[i], comm_, stream_));
@@ -631,7 +593,7 @@ class CudaBackend {
         size_t blocks = (n + kEwThreads - 1) / kEwThreads;
         const size_t cap = (size_t)num_sms_ * 16;
         if (blocks > cap) blocks = cap;
-        before(KK_EW);
+        before(lsted::KK_EW);
         rect_kernel<T><<<(int)blocks, kEwThreads, 0, stream_>>>(a);
         after();
     }
@@ -669,8 +631,7 @@ class CudaBackend {
         p2p_rank_ = rank; p2p_world_ = world; p2p_epoch_ = 0;
     }
     bool p2p_ready(const lsted::ConvGeom& g, int cplx_bytes) const {
-        return p2p_world_ > 1 && use_fast_ &&
-               (cplx_bytes == 8 ? plan_fits_cols<Plan2160f>(g) : plan_fits_cols<Plan2160d>(g));
+        return p2p_world_ > 1 && sw.fast_path && lsted::fast_plan_fits_cols(g, cplx_bytes);
     }
     template <typename T> void p2p_fill(lsted::ColArgs<T>& a) {
         a.p2p_world = p2p_world_; a.p2p_rank = p2p_rank_; a.p2p_epoch = ++p2p_epoch_;
@@ -683,24 +644,18 @@ class CudaBackend {
     }
     // blocks counted on this rank so far = epoch * nxb
     void p2p_wait(int nxb) {
-        before(KK_EW);
+        before(lsted::KK_EW);
         p2p_wait_kernel<<<1, 32, 0, stream_>>>(p2p_done_[p2p_rank_], p2p_epoch_ * (unsigned)nxb);
         after();
     }
     void zero_bytes(void* p, size_t n) { CUDA_CHECK(cudaMemsetAsync(p, 0, n, stream_)); }
-    // centred real OTFs are read by the compile-time column kernels only
-    bool real_otf_supported(const lsted::ConvGeom& g, int cplx_bytes) const {
-        return use_fast_ && real_otf_ &&
-               (cplx_bytes == 8 ? plan_fits_cols<Plan2160f>(g) : plan_fits_cols<Plan2160d>(g));
-    }
     template <typename T> void otf_center(const lsted::OtfCenterArgs<T>& a0) {
         lsted::OtfCenterArgs<T> a = a0;   // the real array is read by the compile-time plans only
-        a.CS = sizeof(T) == 4 ? (int)Plan2160f::CS : (int)Plan2160d::CS;
-        before(KK_EW);
+        a.CS = (int)lsted::PlanFor<T>::type::CS;
+        before(lsted::KK_EW);
         otf_center_kernel<T><<<num_sms_ * 8, 256, 0, stream_>>>(a);
         after();
     }
-    void set_real_otf(bool on) { real_otf_ = on; }
     void fill_double(double* p, size_t n, double v) {
         if (v != 0.0) { lsted::ApiError e; e.code = LSTED_ERR_ARG; e.msg = "fill_double: zero only"; throw e; }
         CUDA_CHECK(cudaMemsetAsync(p, 0, n * sizeof(double), stream_));
@@ -740,7 +695,6 @@ class CudaBackend {
         return ms;
     }
     void set_profile(bool on) { profile_ = on; }
-    void set_k_split(bool on) { k_split_ = on; }
     void set_nvls_probe(bool on) { nvls_probe_ = on; }
     void set_nvls_shape(int ctas, int threads) { if (ctas >= 0) nvls_ctas_ = ctas; if (threads > 0) nvls_threads_ = threads; }
     // ---- CUDA graphs: the steady RL iteration replayed as one driver call (engine.h) ----
@@ -764,17 +718,13 @@ class CudaBackend {
     }
     void graph_launch(void* exec) { CUDA_CHECK(cudaGraphLaunch((cudaGraphExec_t)exec, stream_)); }
     void graph_destroy(void* exec) { if (exec) cudaGraphExecDestroy((cudaGraphExec_t)exec); }
-    void set_fast_path(bool on) { use_fast_ = on; }
-    void set_row_dual(bool on) { row_dual_ = on; }
-    void set_row_plan2(bool on) { row_plan2_ = on; }
     // row CTAs resident at once (4 per SM): prefetch for the CTA one wave ahead
-    int row_prefetch_distance() const { return prefetch_ ? (num_sms_ * prefetch_quarters_) : 0; }
+    int row_prefetch_distance() const { return sw.prefetch ? (num_sms_ * prefetch_quarters_) : 0; }
     // ROW_FINAL has few CTAs (one image): its prefetch must reach past everything resident
     // (4 CTAs per SM) to be of any use -- measured best at 6 CTAs per SM ahead
     int row_final_prefetch_distance() const {
-        return prefetch_ ? num_sms_ * (prefetch_final_quarters_ > 0 ? prefetch_final_quarters_ : prefetch_quarters_) : 0;
+        return sw.prefetch ? num_sms_ * (prefetch_final_quarters_ > 0 ? prefetch_final_quarters_ : prefetch_quarters_) : 0;
     }
-    void set_prefetch(bool on) { prefetch_ = on; }
     void profile_reset() {
         profile_drain();
         memset(prof_ms_, 0, sizeof(prof_ms_));
@@ -797,75 +747,6 @@ class CudaBackend {
         CUDA_CHECK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         have = smem;
     }
-    // ---- fast path (compile-time plans) ----
-    static int fast_cols(int L, int cplx_bytes) {
-        if (L == Plan2160f::L) return cplx_bytes == 8 ? (int)Plan2160f::C : (int)Plan2160d::C;
-        return 0;
-    }
-    template <class P> static bool plan_fits_rows(const lsted::ConvGeom& g) {
-        return g.Lx == P::L && g.C == P::C;
-    }
-    template <class P> static bool plan_fits_cols(const lsted::ConvGeom& g) {
-        return g.Ly == P::L && g.C == P::C;
-    }
-    template <int MODE, class P> void launch_row_fast(int grid, const lsted::RowArgs<typename P::T>& a,
-                                                      int kind) {
-        const size_t smem = lsted::fast_row_smem_bytes<P>(MODE);
-        // fp32 kernels that index pixels have an instance with the headline geometry folded in
-        const bool fixed = sizeof(typename P::T) == 4 && MODE != lsted::ROW_FWD &&
-                           a.g.Nx == (int)RowGeom2048::NX && a.g.sx == (int)RowGeom2048::SX && a.g.Ny % 2 == 0;
-        const bool fixed_c = sizeof(typename P::T) == 4 && MODE != lsted::ROW_FWD &&
-                             a.g.Nx == (int)RowGeom2048c::NX && a.g.sx == 0 && a.g.Ny % 2 == 0;   // centred OTFs
-        ensure_smem(row_fast_kernel<MODE, P>, smem);
-        if (sizeof(typename P::T) == 4) {
-            ensure_smem(row_fast_kernel<MODE, P, RowGeom2048>, smem);
-            ensure_smem(row_fast_kernel<MODE, P, RowGeom2048c>, smem);
-        }
-        // the plan's own pairs-per-CTA decides the grid (the generic geometry may differ)
-        const int fast_grid = a.nimg * ((((a.g.Ny + 1) / 2) + P::PR - 1) / P::PR);
-        (void)grid;
-        if (launch_row_fast_tma<MODE, P>(fast_grid, a, kind, smem, fixed, fixed_c)) return;
-        before(kind);
-        if (fixed) row_fast_kernel<MODE, P, RowGeom2048><<<fast_grid, P::ROW_THREADS, smem, stream_>>>(a);
-        else if (fixed_c) row_fast_kernel<MODE, P, RowGeom2048c><<<fast_grid, P::ROW_THREADS, smem, stream_>>>(a);
-        else row_fast_kernel<MODE, P><<<fast_grid, P::ROW_THREADS, smem, stream_>>>(a);
-        after();
-    }
-    // spectrum chunks by tensor-map bulk copies (fp32, one pair per CTA, ROW_MID / ROW_FINAL)
-    template <int MODE, class P>
-    typename std::enable_if<(sizeof(typename P::T) == 4 && P::PR == 1 &&
-                             (MODE == lsted::ROW_MID || MODE == lsted::ROW_FINAL)), bool>::type
-    launch_row_fast_tma(int fast_grid, const lsted::RowArgs<typename P::T>& a, int kind, size_t smem,
-                        bool fixed, bool fixed_c) {
-        if (!a.tmap_in || !a.tmap_out || !row_tma_) return false;
-        // "lean" ROW_MID: measurement rows staged in the first exchange buffer, two buffers, one
-        // more CTA per SM (bulk copies: the rows must be 16-byte multiples, 16-byte aligned)
-        if (row_tma_ == 2 && (a.g.Nx * sizeof(typename P::T)) % 16 == 0 && ((size_t)a.aux & 15) == 0 &&
-            (MODE == lsted::ROW_MID || ((size_t)a.real_out & 15) == 0)) {
-            const size_t lean = lsted::fast_row_smem_bytes<P>(MODE, true);
-            launch_row_tma_variant<MODE, P, 2>(fast_grid, a, kind, lean, fixed, fixed_c);
-        } else {
-            launch_row_tma_variant<MODE, P, 1>(fast_grid, a, kind, smem, fixed, fixed_c);
-        }
-        return true;
-    }
-    template <int MODE, class P, int TMA>
-    void launch_row_tma_variant(int fast_grid, const lsted::RowArgs<typename P::T>& a, int kind, size_t smem,
-                                bool fixed, bool fixed_c) {
-        ensure_smem(row_fast_kernel<MODE, P, lsted::RowGeomRuntime, TMA>, smem);
-        ensure_smem(row_fast_kernel<MODE, P, RowGeom2048, TMA>, smem);
-        ensure_smem(row_fast_kernel<MODE, P, RowGeom2048c, TMA>, smem);
-        before(kind);
-        if (fixed) row_fast_kernel<MODE, P, RowGeom2048, TMA><<<fast_grid, P::ROW_THREADS, smem, stream_>>>(a);
-        else if (fixed_c) row_fast_kernel<MODE, P, RowGeom2048c, TMA><<<fast_grid, P::ROW_THREADS, smem, stream_>>>(a);
-        else row_fast_kernel<MODE, P, lsted::RowGeomRuntime, TMA><<<fast_grid, P::ROW_THREADS, smem, stream_>>>(a);
-        after();
-    }
-    template <int MODE, class P>
-    typename std::enable_if<!(sizeof(typename P::T) == 4 && P::PR == 1 &&
-                              (MODE == lsted::ROW_MID || MODE == lsted::ROW_FINAL)), bool>::type
-    launch_row_fast_tma(int, const lsted::RowArgs<typename P::T>&, int, size_t, bool, bool) { return false; }
-
     // CUtensorMap (in global memory) of a row-spectrum array: [nimg][nxb][rows_e * C * 2 floats],
     // box = {floats of one pair chunk, kTmaBoxBlocks, 1}.  Returns 0 when tensor maps are unavailable.
     void* make_spec_tmap(void* base, int rows_e, int nxb, int C, int nimg, int chunk_floats) {
@@ -897,156 +778,77 @@ class CudaBackend {
         CUDA_CHECK(cudaStreamSynchronize(stream_));
         return d;
     }
-    bool row_tma_supported(const lsted::ConvGeom& g, int cplx_bytes) const {
-        return use_fast_ && row_tma_ && cplx_bytes == 8 && plan_fits_rows<Plan2160f>(g) && Plan2160f::PR == 1 &&
-               g.nxb >= lsted::kTmaBoxBlocks && g.nxb <= 2 * lsted::kTmaBoxBlocks &&
-               (g.nxb - lsted::kTmaBoxBlocks) % 2 == 0;   // two boxes cover the blocks, 128-byte aligned in smem
+    // ---- launches: dispatch.h chooses the kernel instance, the executors below run it ----
+    template <int MODE, typename T> void launch_row(int grid, const lsted::RowArgs<T>& a) {
+        lsted::run_row<MODE>(*this, lsted::select_row<MODE>(grid, a, sw), a);
     }
-    void set_row_tma(int v) { row_tma_ = v; }
-    template <int MODE, class P> void launch_col_fast(int grid, const lsted::ColArgs<typename P::T>& a,
-                                                      int kind) {
-        const size_t smem = lsted::fast_col_smem_bytes<P>();
-        const bool fixed = sizeof(typename P::T) == 4 && a.g.Ny == (int)ColGeom2048::NY &&
-                           a.g.sy == (int)ColGeom2048::SY && a.rows_in == a.g.Ny;
-        ensure_smem(col_fast_kernel<MODE, P>, smem);
-        if (sizeof(typename P::T) == 4) ensure_smem(col_fast_kernel<MODE, P, ColGeom2048>, smem);
-        if (MODE == lsted::COL_HT && a.p2p_world > 1) {
-            ensure_smem(col_ht_p2p_kernel<P, false>, smem);
-            ensure_smem(col_ht_p2p_kernel<P, true>, smem);
-            const int ncta = grid < num_sms_ ? grid : num_sms_;
-            before(kind);
-            if (a.otf_real) col_ht_p2p_kernel<P, true><<<ncta, P::COL_THREADS, smem, stream_>>>(a);
-            else col_ht_p2p_kernel<P, false><<<ncta, P::COL_THREADS, smem, stream_>>>(a);
-            after();
-            return;
-        }
-        if (a.otf_real) {   // centred real OTFs
-            const bool fixed_c = sizeof(typename P::T) == 4 && a.g.Ny == (int)ColGeom2048c::NY &&
-                                 a.g.sy == 0 && a.rows_in == a.g.Ny;
-            if (launch_col_sub<MODE, P>(grid, a, kind, fixed_c)) return;
-            ensure_smem(col_fast_kernel<MODE, P, lsted::ColGeomRuntime, true>, smem);
-            if (sizeof(typename P::T) == 4) ensure_smem(col_fast_kernel<MODE, P, ColGeom2048c, true>, smem);
-            before(kind);
-            if (fixed_c) col_fast_kernel<MODE, P, ColGeom2048c, true><<<grid, P::COL_THREADS, smem, stream_>>>(a);
-            else col_fast_kernel<MODE, P, lsted::ColGeomRuntime, true><<<grid, P::COL_THREADS, smem, stream_>>>(a);
-            after();
-            return;
-        }
-        before(kind);
-        if (fixed) col_fast_kernel<MODE, P, ColGeom2048><<<grid, P::COL_THREADS, smem, stream_>>>(a);
-        else col_fast_kernel<MODE, P><<<grid, P::COL_THREADS, smem, stream_>>>(a);
+    template <int MODE, typename T> void launch_col(int grid, const lsted::ColArgs<T>& a) {
+        const lsted::DeviceShape dev = {num_sms_, g_live_backends, num_sms_};   // split up to the SM count
+        lsted::run_col<MODE>(*this, lsted::select_col<MODE>(grid, a, sw, dev), a);
+    }
+    template <int MODE, typename T> void row_generic(const lsted::RowChoice& c, const lsted::RowArgs<T>& a) {
+        const size_t smem = lsted::row_smem_bytes(a.g, (int)sizeof(lsted::cplx<T>));
+        ensure_smem(row_kernel<MODE, T>, smem);
+        before(c.kind);
+        row_kernel<MODE, T><<<c.grid, kRowThreads, smem, stream_>>>(a);
         after();
     }
-    // plans with sub-blocks (CS < C): NSUB CTAs per column block, two resident per SM
-    template <int MODE, class P>
-    typename std::enable_if<(P::CS < P::C), bool>::type
-    launch_col_sub(int grid, const lsted::ColArgs<typename P::T>& a, int kind, bool fixed_c) {
-        if (!col_sub_) return false;
-        const size_t smem = lsted::fast_col_sub_smem_bytes<P>();
-        ensure_smem(col_sub_kernel<MODE, P>, smem);
-        ensure_smem(col_sub_kernel<MODE, P, ColGeom2048c>, smem);
-        before(kind);
-        if (fixed_c) col_sub_kernel<MODE, P, ColGeom2048c><<<grid * P::NSUB, P::SUB_THREADS, smem, stream_>>>(a);
-        else col_sub_kernel<MODE, P><<<grid * P::NSUB, P::SUB_THREADS, smem, stream_>>>(a);
+    template <int MODE, class P, class G, int TMA>
+    void row_fast(const lsted::RowChoice& c, const lsted::RowArgs<typename P::T>& a) {
+        const size_t smem = lsted::fast_row_smem_bytes<P>(MODE, TMA == 2);
+        ensure_smem(row_fast_kernel<MODE, P, G, TMA>, smem);
+        before(c.kind);
+        row_fast_kernel<MODE, P, G, TMA><<<c.grid, P::ROW_THREADS, smem, stream_>>>(a);
         after();
-        return true;
     }
-    template <int MODE, class P>
-    typename std::enable_if<!(P::CS < P::C), bool>::type
-    launch_col_sub(int, const lsted::ColArgs<typename P::T>&, int, bool) { return false; }
-    void set_col_sub(bool on) { col_sub_ = on; }
-    template <int MODE> void launch_row2(const lsted::RowArgs<float>& a, int kind) {
-        typedef Plan2160f2 P;
+    // the two-pass and the dual-pair row kernels prefetch one wave of their own CTAs ahead
+    template <int MODE, class P> void row2(const lsted::RowChoice& c, const lsted::RowArgs<float>& a) {
         const size_t smem = lsted::fast_row2_smem_bytes<P>(MODE);
         ensure_smem(row2_fast_kernel<MODE, P>, smem);
         lsted::RowArgs<float> b = a;
         if (b.prefetch_ahead > 0) b.prefetch_ahead = num_sms_ * LSTED_ROW2_CTAS;
-        const int fast_grid = a.nimg * ((((a.g.Ny + 1) / 2) + P::PR - 1) / P::PR);
-        before(kind);
-        row2_fast_kernel<MODE, P><<<fast_grid, P::ROW_THREADS, smem, stream_>>>(b);
+        before(c.kind);
+        row2_fast_kernel<MODE, P><<<c.grid, P::ROW_THREADS, smem, stream_>>>(b);
         after();
     }
-    template <int MODE> bool try_fast_row(int grid, const lsted::RowArgs<float>& a, int kind) {
-        if (!plan_fits_rows<Plan2160f>(a.g)) return false;
-        if (row_plan2_) { launch_row2<MODE>(a, kind); return true; }
-        if (MODE == lsted::ROW_MID && row_dual_ && a.g.Ny % 4 == 0) {
-            typedef lsted::RowDual<Plan2160f> D;
-            const size_t smem = D::smem_bytes();
-            ensure_smem(row_mid_dual_kernel<Plan2160f>, smem);
-            lsted::RowArgs<float> b = a;
-            if (b.prefetch_ahead > 0) b.prefetch_ahead = num_sms_ * 2;   // two CTAs per SM
-            before(kind);
-            row_mid_dual_kernel<Plan2160f><<<a.nimg * (a.g.Ny / 4), D::THREADS, smem, stream_>>>(b);
-            after();
-            return true;
-        }
-        launch_row_fast<MODE, Plan2160f>(grid, a, kind);
-        return true;
-    }
-    template <int MODE> bool try_fast_row(int grid, const lsted::RowArgs<double>& a, int kind) {
-        if (!plan_fits_rows<Plan2160d>(a.g)) return false;
-        launch_row_fast<MODE, Plan2160d>(grid, a, kind);
-        return true;
-    }
-    template <int MODE> bool try_fast_col(int grid, const lsted::ColArgs<float>& a, int kind) {
-        if (MODE == lsted::COL_OTF || !plan_fits_cols<Plan2160f>(a.g)) return false;
-        launch_col_fast<MODE == lsted::COL_OTF ? lsted::COL_H : MODE, Plan2160f>(grid, a, kind);
-        return true;
-    }
-    template <int MODE> bool try_fast_col(int grid, const lsted::ColArgs<double>& a, int kind) {
-        if (MODE == lsted::COL_OTF || !plan_fits_cols<Plan2160d>(a.g)) return false;
-        launch_col_fast<MODE == lsted::COL_OTF ? lsted::COL_H : MODE, Plan2160d>(grid, a, kind);
-        return true;
-    }
-
-    template <int MODE, typename T> void launch_row(int grid, const lsted::RowArgs<T>& a) {
-        if (grid <= 0) return;
-        {
-            const int kind0 = MODE == lsted::ROW_FWD ? KK_ROW_FWD
-                            : MODE == lsted::ROW_INV_STORE ? KK_ROW_INV_STORE
-                            : MODE == lsted::ROW_INV_SIM ? KK_ROW_INV_SIM
-                            : MODE == lsted::ROW_MID ? KK_ROW_MID : KK_ROW_FINAL;
-            if (use_fast_ && try_fast_row<MODE>(grid, a, kind0)) return;
-        }
-        const size_t smem = lsted::row_smem_bytes(a.g, (int)sizeof(lsted::cplx<T>));
-        ensure_smem(row_kernel<MODE, T>, smem);
-        const int kind = MODE == lsted::ROW_FWD ? KK_ROW_FWD
-                       : MODE == lsted::ROW_INV_STORE ? KK_ROW_INV_STORE
-                       : MODE == lsted::ROW_INV_SIM ? KK_ROW_INV_SIM
-                       : MODE == lsted::ROW_MID ? KK_ROW_MID : KK_ROW_FINAL;
-        before(kind);
-        row_kernel<MODE, T><<<grid, kRowThreads, smem, stream_>>>(a);
+    template <class P> void row_mid_dual(const lsted::RowChoice& c, const lsted::RowArgs<float>& a) {
+        typedef lsted::RowDual<P> D;
+        ensure_smem(row_mid_dual_kernel<P>, D::smem_bytes());
+        lsted::RowArgs<float> b = a;
+        if (b.prefetch_ahead > 0) b.prefetch_ahead = num_sms_ * 2;   // two CTAs per SM
+        before(c.kind);
+        row_mid_dual_kernel<P><<<c.grid, D::THREADS, D::smem_bytes(), stream_>>>(b);
         after();
     }
-    template <int MODE, typename T> void launch_col(int grid, const lsted::ColArgs<T>& a) {
-        if (grid <= 0) return;
-        {
-            const int kind0 = MODE == lsted::COL_OTF ? KK_COL_OTF : MODE == lsted::COL_H ? KK_COL_H : KK_COL_HT;
-            if (use_fast_ && try_fast_col<MODE>(grid, a, kind0)) return;
-        }
-        const size_t smem = lsted::col_smem_bytes(a.g, (int)sizeof(lsted::cplx<T>),
-                                                  MODE == lsted::COL_OTF ? 2 : 3);
-        if (smem > lsted::kSmemLimit) {
-            lsted::ApiError e; e.code = LSTED_ERR_ARG;
-            e.msg = "generic column kernel does not fit in shared memory for this geometry";
-            throw e;
-        }
+    template <int MODE, typename T> void col_generic(const lsted::ColChoice& c, const lsted::ColArgs<T>& a) {
+        const size_t smem = lsted::col_smem_bytes(a.g, (int)sizeof(lsted::cplx<T>), MODE == lsted::COL_OTF ? 2 : 3);
         ensure_smem(col_kernel<MODE, T>, smem);
-        const int kind = MODE == lsted::COL_OTF ? KK_COL_OTF : MODE == lsted::COL_H ? KK_COL_H : KK_COL_HT;
-        const int threads = sizeof(T) == 4 ? kColThreads32 : kColThreads64;
-        if (MODE == lsted::COL_H && a.K > 1 && k_split_ && 2 * grid <= num_sms_ && g_live_backends <= 2) {
-            // a small frame (the reference's 128^2 objects: 25 column blocks): the K + 1 dependent
-            // transforms of a block are the latency of this launch; spread the orientations over
-            // the idle SMs, every CTA repeating the forward transform
-            lsted::ColArgs<T> b = a;
-            b.k_split = num_sms_ / grid < a.K ? num_sms_ / grid : a.K;
-            before(kind);
-            col_kernel<MODE, T><<<grid * b.k_split, threads, smem, stream_>>>(b);
-            after();
-            return;
-        }
-        before(kind);
-        col_kernel<MODE, T><<<grid, threads, smem, stream_>>>(a);
+        before(c.kind);
+        col_kernel<MODE, T><<<c.grid, sizeof(T) == 4 ? kColThreads32 : kColThreads64, smem, stream_>>>(a);
+        after();
+    }
+    template <int MODE, class P, class G, bool RO>
+    void col_fast(const lsted::ColChoice& c, const lsted::ColArgs<typename P::T>& a) {
+        const size_t smem = lsted::fast_col_smem_bytes<P>();
+        ensure_smem(col_fast_kernel<MODE, P, G, RO>, smem);
+        before(c.kind);
+        col_fast_kernel<MODE, P, G, RO><<<c.grid, P::COL_THREADS, smem, stream_>>>(a);
+        after();
+    }
+    template <int MODE, class P, class G>
+    void col_sub(const lsted::ColChoice& c, const lsted::ColArgs<typename P::T>& a) {
+        const size_t smem = lsted::fast_col_sub_smem_bytes<P>();
+        ensure_smem(col_sub_kernel<MODE, P, G>, smem);
+        before(c.kind);
+        col_sub_kernel<MODE, P, G><<<c.grid, P::SUB_THREADS, smem, stream_>>>(a);
+        after();
+    }
+    // persistent: at most one CTA per SM, each walks several column blocks
+    template <class P, bool RO> void col_ht_p2p(const lsted::ColChoice& c, const lsted::ColArgs<typename P::T>& a) {
+        const size_t smem = lsted::fast_col_smem_bytes<P>();
+        ensure_smem(col_ht_p2p_kernel<P, RO>, smem);
+        before(c.kind);
+        col_ht_p2p_kernel<P, RO><<<c.grid < num_sms_ ? c.grid : num_sms_, P::COL_THREADS, smem, stream_>>>(a);
         after();
     }
     template <int OP, typename T> void ew(const lsted::EwArgs<T>& a) {
@@ -1054,7 +856,7 @@ class CudaBackend {
         size_t blocks = (a.n + kEwThreads - 1) / kEwThreads;
         const size_t cap = (size_t)num_sms_ * 16;
         if (blocks > cap) blocks = cap;
-        before(KK_EW);
+        before(lsted::KK_EW);
         ew_kernel<OP, T><<<(int)blocks, kEwThreads, 0, stream_>>>(a);
         after();
     }
@@ -1063,7 +865,7 @@ class CudaBackend {
         const size_t n = (size_t)a.Ny * a.Nx;
         if (n == 0) return;
         const size_t blocks = (n + kEwThreads - 1) / kEwThreads;   // one bin per thread: O(N) work each
-        before(KK_EW);
+        before(lsted::KK_EW);
         dft_direct_kernel<PASS, T><<<(unsigned)blocks, kEwThreads, 0, stream_>>>(a);
         after();
     }
@@ -1073,7 +875,7 @@ class CudaBackend {
         size_t blocks = (n + kEwThreads - 1) / kEwThreads;
         const size_t cap = (size_t)num_sms_ * 16;
         if (blocks > cap) blocks = cap;
-        before(KK_EW);
+        before(lsted::KK_EW);
         win_kernel<OP, T><<<(int)blocks, kEwThreads, 0, stream_>>>(a);
         after();
     }
@@ -1102,7 +904,7 @@ class CudaBackend {
         const size_t smem = lsted::col_smem_bytes(a.g, (int)sizeof(lsted::cplx<T>), 2);
         ensure_smem(col_kernel<lsted::COL_LOGMAG, T>, smem);
         const int threads = sizeof(T) == 4 ? kColThreads32 : kColThreads64;
-        before(KK_EW);
+        before(lsted::KK_EW);
         col_kernel<lsted::COL_LOGMAG, T><<<grid, threads, smem, stream_>>>(a);
         after();
     }
@@ -1112,7 +914,7 @@ class CudaBackend {
     }
     double sum(const double* x, size_t n, double* partial) {
         const int blocks = 1024;
-        before(KK_EW);
+        before(lsted::KK_EW);
         sum_partial_kernel<<<blocks, 256, 0, stream_>>>(x, n, partial);
         sum_final_kernel<<<1, 256, 0, stream_>>>(partial, blocks);
         after();
@@ -1134,8 +936,7 @@ class CudaBackend {
     bool nvls_have_mc_ = false, nvls_bound_ = false;
     int nvls_ctas_ = 0, nvls_threads_ = 512;   // options "nvls_ctas" / "nvls_threads" (tuning)
     bool nvls_probe_ = false;                  // option "nvls_probe": barriers only (timing; results are wrong)
-    bool k_split_ = true;                      // option "k_split": orientations of small frames over idle SMs (col_h)
-    bool profile_, use_fast_;
+    bool profile_;
     bool graph_ = getenv("LSTED_GRAPH") ? atoi(getenv("LSTED_GRAPH")) != 0 : true;   // A/B switch, option "graph"
     std::map<void*, size_t> sizes_;   // live allocations (for lsted_deconv_info)
     std::map<const void*, size_t> smem_cfg_;   // kernels whose dynamic shared-memory limit is raised
@@ -1144,19 +945,10 @@ class CudaBackend {
     void* p2p_spec_[lsted::kMaxPeers]; unsigned* p2p_done_[lsted::kMaxPeers];
     std::vector<void*> p2p_opened_;
     int p2p_rank_ = 0, p2p_world_ = 1; unsigned p2p_epoch_ = 0;
-    bool real_otf_ = true;
-    bool col_sub_ = true;     // sub-block column CTAs (2 per SM) where the plan has them
-    int row_tma_ = 2;   // 0 off, 1 tensor-map spectrum copies, 2 also the two-buffer ROW_MID (6 CTAs/SM)
-    bool prefetch_ = true;
     int prefetch_quarters_ = 1;   // row-kernel L2 prefetch distance in CTAs per SM.  With per-thread
                                   // loads it was worth 14 % of row_mid; with the TMA-staged kernels
                                   // it hardly matters for row_mid (1: 0.196, 2: 0.197, 4: 0.199, 8: 0.213 ms)
     int prefetch_final_quarters_ = 6;   // ROW_FINAL (1024 CTAs, 592 resident): 2: 0.0271, 6: 0.0234 ms
-    // two-pass 48 x 45 row kernels (fp32): 35 % fewer warp instructions and half the shared-memory
-    // wavefronts, but 0.334 ms vs 0.283 ms for ROW_MID: 4792 straight-line instructions run by
-    // 9 warps per SM stall on instruction fetch (ncu: no_inst 32 %).  Kept behind this switch.
-    bool row_plan2_ = false;
-    bool row_dual_ = false;   // measured: 0.326 ms vs 0.311 ms for the single-pair kernel (L1TEX-bound either way)
     ncclComm_t comm_ = 0;
     cudaEvent_t t0_, t1_;
     int num_sms_;

@@ -10,15 +10,16 @@
 #include <stdlib.h>
 #include <string.h>
 #include <new>
+#include <initializer_list>
 #include <string>
 #include <vector>
-#include <type_traits>
 #include "../../include/lsted.h"
 #include "../../rescan_line_sted_b200/csrc/engine.h"
 #include "../../rescan_line_sted_b200/csrc/tiled.h"
 #include "../../rescan_line_sted_b200/csrc/conv_fast.cuh"
 #include "../../rescan_line_sted_b200/csrc/ew_bodies.cuh"
 #include "../../rescan_line_sted_b200/csrc/psf_kernels.cuh"
+#include "../../rescan_line_sted_b200/csrc/dispatch.h"
 
 namespace lsted {
 struct ApiError { int code; std::string msg; };
@@ -38,18 +39,6 @@ struct HostCtx {
     }
     template <class R, class F> void phase_nosync(R* regs, F f) { phase(regs, f); }
 };
-
-typedef lsted::FastPlan<float, 16, 9, 15, 144, 4, 1, 2> Plan2160f;
-#ifndef LSTED_FP64_PR
-#define LSTED_FP64_PR 1   // row pairs per CTA of the fp64 plan (A/B at build time; 2: row_mid +13 %)
-#endif
-#ifndef LSTED_FP64_CS
-#define LSTED_FP64_CS 1   // columns per column CTA of the fp64 plan (1 of 2: sub-block CTAs; 2: col_h +15 %, col_ht +35 %)
-#endif
-typedef lsted::FastPlan<double, 16, 9, 15, 144, 2, LSTED_FP64_PR, LSTED_FP64_CS> Plan2160d;
-template <typename T> struct PlanFor;
-template <> struct PlanFor<float> { typedef Plan2160f type; };
-template <> struct PlanFor<double> { typedef Plan2160d type; };
 
 typedef void (*allreduce_cb)(double* buf, size_t n);
 typedef void (*broadcast_cb)(double* buf, size_t n, int root);
@@ -76,19 +65,24 @@ extern "C" int emul_row_tma_launches(void) { return g_row_tma_launches; }
 extern "C" int emul_real_otf_launches(void) { return g_real_otf_launches; }
 extern "C" int emul_row2_launches(void) { return g_row2_launches; }
 extern "C" int emul_dual_launches(void) { return g_dual_launches; }
+// Every row / column launch's choice (dispatch.h), kLogInts per launch: kernel kind, variant,
+// geometry, TMA level, real OTFs, grid, CTAs per column block.  Copies the records from `first`
+// on (at most `cap`) and returns how many there are.
+enum { kLogInts = 7 };
+static std::vector<int> g_dispatch_log;
+extern "C" int emul_dispatch_log(int first, int* out, int cap) {
+    const int n = (int)g_dispatch_log.size() / kLogInts;
+    for (int i = first; i < n && i - first < cap; ++i)
+        memcpy(out + (size_t)(i - first) * kLogInts, &g_dispatch_log[(size_t)i * kLogInts], sizeof(int) * kLogInts);
+    return n;
+}
+static void log_choice(std::initializer_list<int> r) { g_dispatch_log.insert(g_dispatch_log.end(), r); }
 
-class HostBackend {
+class HostBackend : public lsted::KernelSelection {
   public:
-    explicit HostBackend(int) : bytes_(0), use_fast_(true) {
-        const char* ro = getenv("LSTED_REAL_OTF");   // same A/B switch as the CUDA backend
-        if (ro) real_otf_ = atoi(ro) != 0;
-    }
-    void set_fast_path(bool on) { use_fast_ = on; }
-    void set_row_dual(bool on) { row_dual_ = on; }
-    void set_row_plan2(bool on) { row_plan2_ = on; }
-    int row_prefetch_distance() const { return 3; }
-    int row_final_prefetch_distance() const { return 5; }
-    void set_prefetch(bool) {}
+    explicit HostBackend(int) : bytes_(0) {}
+    int row_prefetch_distance() const { return sw.prefetch ? 3 : 0; }
+    int row_final_prefetch_distance() const { return sw.prefetch ? 5 : 0; }
     // NVLS needs the NVSwitch: never available on the CPU replay
     static bool nvls_device_supported(int) { return false; }
     bool nvls_ready(const void*) const { return false; }
@@ -99,7 +93,6 @@ class HostBackend {
     template <typename T> void nvls_allreduce(T*, size_t) { throw std::string("NVLS: GPU only"); }
     void set_nvls_shape(int, int) {}
     void set_nvls_probe(bool) {}
-    void set_k_split(bool) {}
     void set_graph(bool) {}
     bool graph_capable() const { return false; }   // captured launches exist on the GPU only
     void graph_begin() {}
@@ -107,10 +100,6 @@ class HostBackend {
     void* graph_end() { return 0; }
     void graph_launch(void*) {}
     void graph_destroy(void*) {}
-    static int fast_cols(int L, int cplx_bytes) {
-        if (L == Plan2160f::L) return cplx_bytes == 8 ? (int)Plan2160f::C : (int)Plan2160d::C;
-        return 0;
-    }
     void activate() {}
     void sync() {}
     void* alloc(size_t bytes) { bytes_ += bytes; return malloc(bytes ? bytes : 1); }
@@ -141,24 +130,14 @@ class HostBackend {
     void fill_double(double* p, size_t n, double v) { for (size_t i = 0; i < n; ++i) p[i] = v; }
     // peer-memory reduction: GPU only (the CPU replay reduces through the callback)
     void zero_bytes(void* p, size_t n) { memset(p, 0, n); }
-    bool real_otf_supported(const lsted::ConvGeom& g, int cplx_bytes) const {
-        return use_fast_ && real_otf_ && g.Ly == Plan2160f::L &&
-               g.C == (cplx_bytes == 8 ? (int)Plan2160f::C : (int)Plan2160d::C);
-    }
     template <typename T> void otf_center(const lsted::OtfCenterArgs<T>& a0) {
         lsted::OtfCenterArgs<T> a = a0;
-        a.CS = (int)PlanFor<T>::type::CS;
+        a.CS = (int)lsted::PlanFor<T>::type::CS;
         for (size_t i = 0; i < a.n; ++i) lsted::otf_center_apply<T>(a, i);
     }
-    void set_real_otf(bool on) { real_otf_ = on; }
     // tensor-map copies: the host replay runs the same staged code path with plain loops
     // (fft_core.cuh); the "descriptor" is just a non-null token
     void* make_spec_tmap(void*, int, int, int, int, int) { return alloc(8); }
-    bool row_tma_supported(const lsted::ConvGeom& g, int cplx_bytes) const {
-        return use_fast_ && row_tma_ && cplx_bytes == 8 && g.Lx == Plan2160f::L && g.C == (int)Plan2160f::C;
-    }
-    void set_row_tma(int v) { row_tma_ = v; }
-    void set_col_sub(bool on) { col_sub_ = on; }
     void p2p_export(void*, void*, void*, char*) { throw std::string("peer memory needs GPUs"); }
     void p2p_attach(int, int, const char*, size_t) { throw std::string("peer memory needs GPUs"); }
     bool p2p_ready(const lsted::ConvGeom&, int) const { return false; }
@@ -172,167 +151,76 @@ class HostBackend {
     }
     void profile_reset() {}
 
+    // ---- launches: dispatch.h chooses as on the GPU; the executors run the CTAs one by one ----
     template <int MODE, typename T> void launch_row(int grid, const lsted::RowArgs<T>& a) {
-        typedef typename PlanFor<T>::type P;
-        if (use_fast_ && row_plan2_ && a.g.Lx == P::L && a.g.C == P::C && launch_row2<MODE>(a)) return;
-        if (use_fast_ && row_dual_ && MODE == lsted::ROW_MID && a.g.Lx == P::L && a.g.C == P::C &&
-            a.g.Ny % 4 == 0 && launch_row_mid_dual(a))
-            return;
-        if (use_fast_ && a.g.Lx == P::L && a.g.C == P::C) {
-            grid = a.nimg * ((((a.g.Ny + 1) / 2) + P::PR - 1) / P::PR);
-#pragma omp parallel
-            {
-                std::vector<lsted::cplx<T> > smem(lsted::fast_row_smem_bytes<P>(MODE) / sizeof(lsted::cplx<T>));
-                std::vector<lsted::RowRegs<P> > regs(P::ROW_THREADS);
-                HostCtx cx;
-                cx.nthreads = P::ROW_THREADS;
-                // same dispatch as the CUDA backend: compile-time geometry for 2048-wide rows
-                const bool fixed = sizeof(T) == 4 && MODE != lsted::ROW_FWD && a.g.Nx == 2048 && a.g.sx == 53 && a.g.Ny % 2 == 0;
-#pragma omp for schedule(dynamic)
-                for (int b = 0; b < grid; ++b) {
-                    if (run_row_tma<MODE, P>(cx, b, a, smem.data(), regs.data())) continue;
-                    if (fixed)
-                        lsted::row_fast_body<MODE, P, HostCtx, lsted::RowGeomFixed<2048, 53> >(
-                            cx, b, a, smem.data(), regs.data());
-                    else
-                        lsted::row_fast_body<MODE, P>(cx, b, a, smem.data(), regs.data());
-                }
-            }
-            return;
-        }
-#pragma omp parallel
-        {
-            std::vector<lsted::cplx<T> > smem((size_t)2 * a.g.PR * a.g.Lpx);
-            HostCtx cx;
-#pragma omp for schedule(dynamic)
-            for (int b = 0; b < grid; ++b) lsted::row_body<MODE, T>(cx, b, a, smem.data());
-        }
-    }
-    template <int MODE, class P>
-    typename std::enable_if<(sizeof(typename P::T) == 4 && P::PR == 1 &&
-                             (MODE == lsted::ROW_MID || MODE == lsted::ROW_FINAL)), bool>::type
-    run_row_tma(HostCtx& cx, int b, const lsted::RowArgs<typename P::T>& a, lsted::cplx<typename P::T>* smem,
-                lsted::RowRegs<P>* regs) {
-        if (!a.tmap_in || !a.tmap_out || !row_tma_) return false;
-        if (b == 0) {
-#pragma omp atomic
-            ++g_row_tma_launches;
-        }
-        if (row_tma_ == 2 && (a.g.Nx * sizeof(typename P::T)) % 16 == 0 && ((size_t)a.aux & 15) == 0 &&
-            (MODE == lsted::ROW_MID || ((size_t)a.real_out & 15) == 0))
-            lsted::row_fast_body<MODE, P, HostCtx, lsted::RowGeomRuntime, 2>(cx, b, a, smem, regs);
-        else
-            lsted::row_fast_body<MODE, P, HostCtx, lsted::RowGeomRuntime, 1>(cx, b, a, smem, regs);
-        return true;
-    }
-    template <int MODE, class P>
-    typename std::enable_if<!(sizeof(typename P::T) == 4 && P::PR == 1 &&
-                              (MODE == lsted::ROW_MID || MODE == lsted::ROW_FINAL)), bool>::type
-    run_row_tma(HostCtx&, int, const lsted::RowArgs<typename P::T>&, lsted::cplx<typename P::T>*,
-                lsted::RowRegs<P>*) { return false; }
-    template <int MODE> bool launch_row2(const lsted::RowArgs<double>&) { return false; }
-    template <int MODE> bool launch_row2(const lsted::RowArgs<float>& a) {
-        typedef lsted::FastPlan2<float, 48, 45, 4, 2> P;
-        const int grid = a.nimg * ((((a.g.Ny + 1) / 2) + P::PR - 1) / P::PR);
-        ++g_row2_launches;
-#pragma omp parallel
-        {
-            std::vector<lsted::cplx<float> > smem(lsted::fast_row2_smem_bytes<P>(MODE) / sizeof(lsted::cplx<float>));
-            std::vector<lsted::Row2Regs<P> > regs(P::ROW_THREADS);
-            HostCtx cx;
-            cx.nthreads = P::ROW_THREADS;
-            const bool fixed = MODE != lsted::ROW_FWD && a.g.Nx == 2048 && a.g.sx == 53 && a.g.Ny % 2 == 0;
-#pragma omp for schedule(dynamic)
-            for (int b = 0; b < grid; ++b) {
-                if (fixed)
-                    lsted::row2_fast_body<MODE, P, HostCtx, lsted::RowGeomFixed<2048, 53> >(
-                        cx, b, a, smem.data(), regs.data());
-                else
-                    lsted::row2_fast_body<MODE, P>(cx, b, a, smem.data(), regs.data());
-            }
-        }
-        return true;
-    }
-    bool launch_row_mid_dual(const lsted::RowArgs<double>&) { return false; }
-    bool launch_row_mid_dual(const lsted::RowArgs<float>& a) {
-        typedef lsted::RowDual<Plan2160f> D;
-        ++g_dual_launches;
-        const int grid = a.nimg * (a.g.Ny / 4);
-#pragma omp parallel
-        {
-            std::vector<lsted::c2> smem(D::smem_bytes() / sizeof(lsted::c2) + 1);
-            std::vector<D::Regs> regs(D::THREADS);
-            HostCtx cx;
-            cx.nthreads = D::THREADS;
-#pragma omp for schedule(dynamic)
-            for (int b = 0; b < grid; ++b)
-                lsted::row_mid_dual_body<Plan2160f>(cx, b, a, (unsigned char*)smem.data(), regs.data());
-        }
-        return true;
+        const lsted::RowChoice c = lsted::select_row<MODE>(grid, a, sw);
+        log_choice({c.kind, (int)c.variant, (int)c.geom, c.tma, 0, c.grid, 1});
+        g_row2_launches += c.variant == lsted::RowVariant::row2;
+        g_dual_launches += c.variant == lsted::RowVariant::row_mid_dual;
+        g_row_tma_launches += c.tma > 0;
+        lsted::run_row<MODE>(*this, c, a);
     }
     template <int MODE, typename T> void launch_col(int grid, const lsted::ColArgs<T>& a) {
-        typedef typename PlanFor<T>::type P;
-        if (use_fast_ && MODE != lsted::COL_OTF && a.g.Ly == P::L && a.g.C == P::C && a.otf_real &&
-            (int)P::CS < (int)P::C && col_sub_) {
-            // sub-block column CTAs (two per SM on the GPU)
-            ++g_col_sub_launches;
-            ++g_real_otf_launches;
-#pragma omp parallel
-            {
-                std::vector<lsted::cplx<T> > smem(lsted::fast_col_sub_smem_bytes<P>() / sizeof(lsted::cplx<T>) + 1);
-                std::vector<lsted::ColRegs<P> > regs(P::SUB_THREADS);
-                HostCtx cx;
-                cx.nthreads = P::SUB_THREADS;
-#pragma omp for schedule(dynamic)
-                for (int b = 0; b < grid * (int)P::NSUB; ++b)
-                    lsted::col_fast_body<(MODE == lsted::COL_OTF ? lsted::COL_H : MODE), P, HostCtx,
-                                         lsted::ColGeomRuntime, true, true>(cx, b, a, smem.data(), regs.data());
-            }
-            return;
-        }
-        if (use_fast_ && MODE != lsted::COL_OTF && a.g.Ly == P::L && a.g.C == P::C) {
-#pragma omp parallel
-            {
-                std::vector<lsted::cplx<T> > smem(lsted::fast_col_smem_bytes<P>() / sizeof(lsted::cplx<T>) + 1);
-                std::vector<lsted::ColRegs<P> > regs(P::COL_THREADS);
-                HostCtx cx;
-                cx.nthreads = P::COL_THREADS;
-                const bool fixed = sizeof(T) == 4 && a.g.Ny == 2048 && a.g.sy == 53 && !a.otf_real;
-                if (a.otf_real) {
-#pragma omp single
-                    ++g_real_otf_launches;
-                }
-#pragma omp for schedule(dynamic)
-                for (int b = 0; b < grid; ++b) {
-                    if (a.otf_real)
-                        lsted::col_fast_body<(MODE == lsted::COL_OTF ? lsted::COL_H : MODE), P, HostCtx,
-                                             lsted::ColGeomRuntime, true>(cx, b, a, smem.data(), regs.data());
-                    else if (fixed)
-                        lsted::col_fast_body<(MODE == lsted::COL_OTF ? lsted::COL_H : MODE), P, HostCtx,
-                                             lsted::ColGeomFixed<2048, 53> >(cx, b, a, smem.data(), regs.data());
-                    else
-                        lsted::col_fast_body<(MODE == lsted::COL_OTF ? lsted::COL_H : MODE), P>(
-                            cx, b, a, smem.data(), regs.data());
-                }
-            }
-            return;
-        }
-        // small frames: the orientations of a column block spread over several "CTAs" like on
-        // the GPU (there: as many as idle SMs allow; here 3, an uneven split of most K)
-        lsted::ColArgs<T> b_args = a;
-        int total = grid;
-        if (MODE == lsted::COL_H && a.K > 1 && grid <= 74) {
-            b_args.k_split = a.K < 3 ? a.K : 3;
-            total = grid * b_args.k_split;
-            ++g_k_split_launches;
-        }
+        // a B200 with one live handle; at most 3 CTAs per column block keeps the split of most K uneven
+        const lsted::DeviceShape dev = {148, 1, 3};
+        const lsted::ColChoice c = lsted::select_col<MODE>(grid, a, sw, dev);
+        log_choice({c.kind, (int)c.variant, (int)c.geom, 0, c.real_otf, c.grid, c.k_split});
+        g_col_sub_launches += c.variant == lsted::ColVariant::fast_sub;
+        g_real_otf_launches += c.variant != lsted::ColVariant::generic && c.real_otf;
+        g_k_split_launches += c.k_split > 1;
+        lsted::run_col<MODE>(*this, c, a);
+    }
+    // the CTAs of one launch, each with its own shared memory and per-thread registers
+    template <class S, class R, class F> void ctas(int grid, size_t smem_bytes, int threads, F body) {
 #pragma omp parallel
         {
-            std::vector<lsted::cplx<T> > smem((size_t)3 * a.g.C * a.g.Lpy);  // (no 227 KB limit here)
+            std::vector<S> smem(smem_bytes / sizeof(S) + 1);
+            std::vector<R> regs(threads);
             HostCtx cx;
+            cx.nthreads = threads;
 #pragma omp for schedule(dynamic)
-            for (int b = 0; b < total; ++b) lsted::col_body<MODE, T>(cx, b, b_args, smem.data());
+            for (int b = 0; b < grid; ++b) body(cx, b, smem.data(), regs.data());
         }
+    }
+    template <int MODE, typename T> void row_generic(const lsted::RowChoice& c, const lsted::RowArgs<T>& a) {
+        ctas<lsted::cplx<T>, char>(c.grid, lsted::row_smem_bytes(a.g, sizeof(lsted::cplx<T>)), 1,
+                                   [&](HostCtx& cx, int b, auto* smem, auto*) { lsted::row_body<MODE, T>(cx, b, a, smem); });
+    }
+    template <int MODE, class P, class G, int TMA>
+    void row_fast(const lsted::RowChoice& c, const lsted::RowArgs<typename P::T>& a) {
+        ctas<lsted::cplx<typename P::T>, lsted::RowRegs<P> >(
+            c.grid, lsted::fast_row_smem_bytes<P>(MODE, TMA == 2), P::ROW_THREADS,
+            [&](HostCtx& cx, int b, auto* smem, auto* regs) { lsted::row_fast_body<MODE, P, HostCtx, G, TMA>(cx, b, a, smem, regs); });
+    }
+    template <int MODE, class P> void row2(const lsted::RowChoice& c, const lsted::RowArgs<float>& a) {
+        ctas<lsted::cplx<float>, lsted::Row2Regs<P> >(
+            c.grid, lsted::fast_row2_smem_bytes<P>(MODE), P::ROW_THREADS,
+            [&](HostCtx& cx, int b, auto* smem, auto* regs) { lsted::row2_fast_body<MODE, P>(cx, b, a, smem, regs); });
+    }
+    template <class P> void row_mid_dual(const lsted::RowChoice& c, const lsted::RowArgs<float>& a) {
+        typedef lsted::RowDual<P> D;
+        ctas<lsted::c2, typename D::Regs>(c.grid, D::smem_bytes(), D::THREADS, [&](HostCtx& cx, int b, auto* smem, auto* regs) {
+            lsted::row_mid_dual_body<P>(cx, b, a, (unsigned char*)smem, regs);
+        });
+    }
+    template <int MODE, typename T> void col_generic(const lsted::ColChoice& c, const lsted::ColArgs<T>& a) {
+        ctas<lsted::cplx<T>, char>(c.grid, lsted::col_smem_bytes(a.g, sizeof(lsted::cplx<T>), MODE == lsted::COL_OTF ? 2 : 3), 1,
+                                   [&](HostCtx& cx, int b, auto* smem, auto*) { lsted::col_body<MODE, T>(cx, b, a, smem); });
+    }
+    template <int MODE, class P, class G, bool RO>
+    void col_fast(const lsted::ColChoice& c, const lsted::ColArgs<typename P::T>& a) {
+        ctas<lsted::cplx<typename P::T>, lsted::ColRegs<P> >(
+            c.grid, lsted::fast_col_smem_bytes<P>(), P::COL_THREADS,
+            [&](HostCtx& cx, int b, auto* smem, auto* regs) { lsted::col_fast_body<MODE, P, HostCtx, G, RO>(cx, b, a, smem, regs); });
+    }
+    template <int MODE, class P, class G>
+    void col_sub(const lsted::ColChoice& c, const lsted::ColArgs<typename P::T>& a) {
+        ctas<lsted::cplx<typename P::T>, lsted::ColRegs<P> >(
+            c.grid, lsted::fast_col_sub_smem_bytes<P>(), P::SUB_THREADS,
+            [&](HostCtx& cx, int b, auto* smem, auto* regs) { lsted::col_fast_body<MODE, P, HostCtx, G, true, true>(cx, b, a, smem, regs); });
+    }
+    template <class P, bool RO> void col_ht_p2p(const lsted::ColChoice&, const lsted::ColArgs<typename P::T>&) {
+        throw std::string("peer memory needs GPUs");
     }
     template <int OP, typename T> void ew(const lsted::EwArgs<T>& a) {
         for (size_t i = 0; i < a.n; ++i) lsted::ew_apply<OP, T>(a, i);
@@ -405,12 +293,6 @@ class HostBackend {
 
   private:
     size_t bytes_;
-    bool use_fast_;
-    bool row_dual_ = false;
-    bool row_plan2_ = false;
-    bool real_otf_ = true;
-    int row_tma_ = 2;
-    bool col_sub_ = true;
 };
 
 #define LSTED_BACKEND HostBackend

@@ -1,7 +1,8 @@
 """Every kernel path the engine dispatches to on the GPU, against the fp64 oracle, and the GPU
 noise field against the textbook sampler, pixel for pixel.
 
-The engine picks its kernels per axis and per launch (lsted_api.cu: launch_row / launch_col):
+The engine picks its kernels per axis and per launch (dispatch.h: select_row / select_col, the
+same functions on the CPU replay, where test_kernel_selection.py pins every case's choices):
 the compile-time 2160 plan when the transform length is 2160 and the column geometry has the
 plan's C, else the generic Stockham kernels with C = 4, 2, 1 columns and PR = 2, 1 row pairs per
 CTA; fixed-geometry instances for 2048-wide images (RowGeom2048 / ColGeom2048 with complex OTFs,
