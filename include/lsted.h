@@ -3,7 +3,8 @@
  * Every entry point returns 0 on success and a non-zero status otherwise;
  * lsted_last_error() then returns a thread-local, human-readable message.
  * All array arguments are HOST pointers to C-contiguous float64 data unless
- * the name says otherwise; the library owns all device memory.  Handles are
+ * the name says otherwise (the _dev entry points take device buffers of float32
+ * or float64); the library owns all device memory it allocates.  Handles are
  * not thread-safe; each owns one CUDA stream.  There is no CPU fallback: a
  * call without a usable CUDA device fails with LSTED_ERR_CUDA.
  *
@@ -204,6 +205,29 @@ int lsted_deconv_set(lsted_deconv* h, int which, int k, const double* in);
 /* H (:567-577): x[Ny][Nx] -> out[K][Ny][Nx];  H_t (:579-594): y[K][Ny][Nx] -> out[Ny][Nx]. */
 int lsted_deconv_H(lsted_deconv* h, const double* x, double* out);
 int lsted_deconv_Ht(lsted_deconv* h, const double* y, double* out, int normalize);
+
+/* ---- the same on DEVICE buffers (e.g. torch.Tensor.data_ptr()), no host round trip ----
+ * Each _dev call mirrors its host twin above (shapes, `which` / `k`, side effects on the
+ * handle); lsted_deconv_simulate after lsted_deconv_upload_object_dev is the device form of
+ * lsted_deconv_create_data.  Buffers are C-contiguous, of element type `dtype`, at least
+ * element-aligned (16-byte alignment takes vector accesses), in device (or managed) memory of
+ * the handle's device.  float32 values enter exactly and leave rounded to nearest once, so a
+ * call gives the bits of the host call fed the same values.
+ * Stream contract: `stream` is a cudaStream_t on the handle's device (NULL: the legacy default
+ * stream), in PyTorch torch.cuda.current_stream().cuda_stream.  The handle's work starts after
+ * everything already enqueued on `stream`; everything enqueued on `stream` later waits for the
+ * call's reads and writes (one event each way), so an input may be freed or reused as soon as
+ * the call returns.  No call blocks the host.  A stream being captured into a CUDA graph is
+ * refused with LSTED_ERR_STATE.  Every argument is checked before anything is enqueued: a bad
+ * dtype, a misaligned pointer, host memory, memory of another device, or a range running past
+ * its allocation fails with LSTED_ERR_ARG.                                                      */
+enum { LSTED_F32 = 32, LSTED_F64 = 64 };   /* element type of caller device buffers */
+int lsted_deconv_get_dev(lsted_deconv* h, int which, int k, void* out, int dtype, void* stream);
+int lsted_deconv_set_dev(lsted_deconv* h, int which, int k, const void* in, int dtype, void* stream);
+int lsted_deconv_upload_object_dev(lsted_deconv* h, const void* object, int dtype, void* stream);
+/* x[Ny][Nx] -> out[K][Ny][Nx];  y[K][Ny][Nx] -> out[Ny][Nx]; x / y and out share `dtype`.    */
+int lsted_deconv_H_dev(lsted_deconv* h, const void* x, void* out, int dtype, void* stream);
+int lsted_deconv_Ht_dev(lsted_deconv* h, const void* y, void* out, int dtype, int normalize, void* stream);
 int lsted_deconv_sync(lsted_deconv* h);
 /* CUDA-event stopwatch on the handle's stream.                                     */
 int lsted_deconv_timer_start(lsted_deconv* h);

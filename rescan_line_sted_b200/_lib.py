@@ -6,6 +6,7 @@ raises RuntimeError with the library's message when CUDA fails.
 """
 import ctypes
 import os
+import sys
 
 import numpy as np
 
@@ -89,6 +90,17 @@ _DECONV_SIGNATURES = {
     'lsted_deconv_ft_error': [ctypes.c_void_p, c_double_p, c_double_p, c_int_p],
     'lsted_deconv_H': [ctypes.c_void_p, c_double_p, c_double_p],
     'lsted_deconv_Ht': [ctypes.c_void_p, c_double_p, c_double_p, ctypes.c_int],
+    # device-buffer twins: (..., pointer(s), dtype 32 | 64, [normalize,] cudaStream_t)
+    'lsted_deconv_get_dev': [ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_void_p,
+                             ctypes.c_int, ctypes.c_void_p],
+    'lsted_deconv_set_dev': [ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_void_p,
+                             ctypes.c_int, ctypes.c_void_p],
+    'lsted_deconv_upload_object_dev': [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int,
+                                       ctypes.c_void_p],
+    'lsted_deconv_H_dev': [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int,
+                           ctypes.c_void_p],
+    'lsted_deconv_Ht_dev': [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int,
+                            ctypes.c_int, ctypes.c_void_p],
     'lsted_deconv_sync': [ctypes.c_void_p],
     'lsted_deconv_timer_start': [ctypes.c_void_p],
     'lsted_deconv_timer_stop': [ctypes.c_void_p,
@@ -172,6 +184,35 @@ def as_f64(a):
     return a, a.ctypes.data_as(c_double_p)
 
 
+def is_tensor(x):
+    """True for a torch.Tensor.  torch is never imported here: a caller that
+    holds a tensor has imported it already."""
+    torch = sys.modules.get('torch')
+    return torch is not None and isinstance(x, torch.Tensor)
+
+
+def check_tensor(t, shape, device, what):
+    """Raise TypeError / ValueError unless `t` is a C-contiguous float32 or
+    float64 CUDA tensor of `shape` (None: any extent) on CUDA device `device`.
+    Everything but the device is checked first, so a CPU tensor shows its other
+    faults too."""
+    import torch
+    if not isinstance(t, torch.Tensor):
+        raise TypeError('%s must be a torch.Tensor, got %s' % (what, type(t).__name__))
+    if t.dtype not in (torch.float32, torch.float64):
+        raise TypeError('%s must be float32 or float64, got %s' % (what, t.dtype))
+    if t.dim() != len(shape) or any(s is not None and s != n for s, n in zip(shape, t.shape)):
+        want = '(%s)' % ', '.join('n' if s is None else str(s) for s in shape)
+        raise ValueError('%s must have shape %s, got %s' % (what, want, tuple(t.shape)))
+    if not t.is_contiguous():
+        raise ValueError('%s must be C-contiguous' % what)
+    if t.device.type != 'cuda':
+        raise ValueError('%s must be a CUDA tensor, got one on %s' % (what, t.device))
+    if t.device.index != device:
+        raise ValueError('%s is on %s, the handle on cuda:%d' % (what, t.device, device))
+    return t
+
+
 _library = None
 
 
@@ -209,6 +250,7 @@ class DeconvHandle:
         self.K, self.ny, self.nx = psfs.shape
         self.Ny, self.Nx = int(image_shape[0]), int(image_shape[1])
         self.precision = precision
+        self.device = int(device)
         self._h = ctypes.c_void_p()
         lib.call('lsted_deconv_create_tiled', ctypes.byref(self._h), device,
                  psfs.ctypes.data_as(c_double_p), self.K, self.ny, self.nx,
@@ -343,6 +385,60 @@ class DeconvHandle:
         out = np.empty((1, self.Ny, self.Nx), dtype=np.float64)
         self.lib.call('lsted_deconv_Ht', self._h, p,
                       out.ctypes.data_as(c_double_p), int(bool(normalize)))
+        return out
+
+    # -- torch.Tensor forms (the _dev entry points): CUDA tensors on the handle's device,
+    # float32 or float64, C-contiguous; ordered on the current torch stream, no host round trip
+    def _stream(self):
+        import torch
+        return ctypes.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+
+    def _image(self, t, nimg, what):
+        return check_tensor(t, (nimg, self.Ny, self.Nx), self.device, what)
+
+    @staticmethod
+    def _dtype_bits(t):
+        return 32 if t.element_size() == 4 else 64
+
+    def get_tensor(self, which, k=0, dtype=None, out=None):
+        """Attribute `which` (PSF k) as a (1, Ny, Nx) tensor of `dtype` (float64 by
+        default), or into `out`."""
+        import torch
+        if out is None:
+            out = torch.empty((1, self.Ny, self.Nx), dtype=dtype or torch.float64,
+                              device=torch.device('cuda', self.device))
+        self._image(out, 1, 'out')
+        self.lib.call('lsted_deconv_get_dev', self._h, which, k, out.data_ptr(),
+                      self._dtype_bits(out), self._stream())
+        return out
+
+    def set_tensor(self, which, k, t):
+        self._image(t, 1, 'the image')
+        self.lib.call('lsted_deconv_set_dev', self._h, which, k, t.data_ptr(),
+                      self._dtype_bits(t), self._stream())
+
+    def upload_object_tensor(self, obj):
+        """Stage an object from a tensor (then simulate(): the device form of create_data)."""
+        self._image(obj, 1, 'the object')
+        self.lib.call('lsted_deconv_upload_object_dev', self._h, obj.data_ptr(),
+                      self._dtype_bits(obj), self._stream())
+
+    def H_tensor(self, x):
+        """(1, Ny, Nx) -> (K, Ny, Nx), dtype of x."""
+        import torch
+        self._image(x, 1, 'x')
+        out = torch.empty((self.K, self.Ny, self.Nx), dtype=x.dtype, device=x.device)
+        self.lib.call('lsted_deconv_H_dev', self._h, x.data_ptr(), out.data_ptr(),
+                      self._dtype_bits(x), self._stream())
+        return out
+
+    def Ht_tensor(self, y, normalize=True):
+        """(K, Ny, Nx) -> (1, Ny, Nx), dtype of y."""
+        import torch
+        self._image(y, self.K, 'y')
+        out = torch.empty((1, self.Ny, self.Nx), dtype=y.dtype, device=y.device)
+        self.lib.call('lsted_deconv_Ht_dev', self._h, y.data_ptr(), out.data_ptr(),
+                      self._dtype_bits(y), int(bool(normalize)), self._stream())
         return out
 
     def sync(self):

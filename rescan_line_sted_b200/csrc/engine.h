@@ -24,6 +24,46 @@ enum ArrayId {
     ARR_NORMALIZATION = 4
 };
 
+// An image crossing the engine's boundary: host float64 (dtype 0, the host entry points) or a
+// caller's device buffer of float32 / float64 (dtype 32 / 64, the _dev entry points).  Either
+// way it passes through the engine's fp64 staging array: one host copy, or one conversion launch
+// (ew_bodies.cuh stage_apply) that rounds like the host path.
+struct ImageRef {
+    void* p;
+    int dtype;
+    ImageRef at(size_t elems) const {
+        ImageRef r = {(char*)p + elems * (dtype == 32 ? 4 : 8), dtype};
+        return r;
+    }
+};
+inline ImageRef host_image(const double* p) {
+    ImageRef r = {(void*)p, 0};
+    return r;
+}
+// caller buffer <-> fp64 staging: one element-wise launch (ew_bodies.cuh stage_apply)
+template <int OP, typename U, class BK> void convert_stage(BK& bk, void* user, double* stage, size_t n) {
+    EwArgs<U> a;
+    memset(&a, 0, sizeof(a));
+    if (OP == EW_TO_STAGE) { a.t1 = (const U*)user; a.d0 = stage; }
+    else { a.t0 = (U*)user; a.d1 = stage; }
+    a.elems = n;
+    a.vec = ((uintptr_t)user & 15) == 0;
+    a.n = stage_items<U>(n, a.vec != 0);
+    bk.template ew<OP, U>(a);
+}
+// stage[0, n) <- src
+template <class BK> void stage_in(BK& bk, double* stage, const ImageRef& src, size_t n) {
+    if (src.dtype == 0) bk.upload(stage, src.p, sizeof(double) * n);
+    else if (src.dtype == 32) convert_stage<EW_TO_STAGE, float>(bk, src.p, stage, n);
+    else convert_stage<EW_TO_STAGE, double>(bk, src.p, stage, n);
+}
+// dst <- stage[0, n); a host destination is complete on return
+template <class BK> void stage_out(BK& bk, const ImageRef& dst, double* stage, size_t n) {
+    if (dst.dtype == 0) bk.download(dst.p, stage, sizeof(double) * n);
+    else if (dst.dtype == 32) convert_stage<EW_FROM_STAGE, float>(bk, dst.p, stage, n);
+    else convert_stage<EW_FROM_STAGE, double>(bk, dst.p, stage, n);
+}
+
 // Precision-independent face of an engine: what the C ABI talks to.
 struct EngineInfo {
     int K, ny, nx, Ny, Nx, Ly, Lx, C, PR, iterations_done;
@@ -36,15 +76,15 @@ class EngineBase {
   public:
     virtual ~EngineBase() {}
     virtual void set_psfs(const double* psfs_host) = 0;
-    virtual void upload_object(const double* obj_host) = 0;
+    virtual void upload_object(const ImageRef& obj) = 0;
     virtual void simulate(double total_brightness, bool rescale, unsigned long long seed) = 0;
     virtual void create_data(const double* obj_host, double total_brightness, bool rescale,
                              unsigned long long seed) = 0;
     virtual void iterate(int n) = 0;
-    virtual void get_array(int id, int k, double* host) = 0;
-    virtual void set_array(int id, int k, const double* host) = 0;
-    virtual void H_host(const double* x, double* out) = 0;
-    virtual void Ht_host(const double* y, double* out, bool normalize) = 0;
+    virtual void get_array(int id, int k, const ImageRef& out) = 0;
+    virtual void set_array(int id, int k, const ImageRef& in) = 0;
+    virtual void H(const ImageRef& x, const ImageRef& out) = 0;                    // out: K images
+    virtual void Ht(const ImageRef& y, const ImageRef& out, bool normalize) = 0;   // y: K images
     virtual void forget_normalization() = 0;
     virtual void reset_estimate() = 0;     // the next iterate() starts from ones (ref:521-522)
     virtual void set_sharding(int rank, int world, int k_offset) = 0;
@@ -209,9 +249,7 @@ template <typename T, class BK> class DeconvEngine : public EngineBase {
     }
 
     // ---- Deconvolver methods ---------------------------------------------
-    void upload_object(const double* obj_host) {
-        bk.upload(object64, obj_host, sizeof(double) * npix);
-    }
+    void upload_object(const ImageRef& obj) { stage_in(bk, object64, obj, npix); }
     // Forward model + shot noise from the object staged by upload_object().
     void simulate(double total_brightness, bool rescale, unsigned long long seed) {
         double s = 1.0;
@@ -224,7 +262,7 @@ template <typename T, class BK> class DeconvEngine : public EngineBase {
     }
     void create_data(const double* obj_host, double total_brightness, bool rescale,
                      unsigned long long seed) {
-        upload_object(obj_host);
+        upload_object(host_image(obj_host));
         simulate(total_brightness, rescale, seed);
     }
     void forget_normalization() { have_norm = false; }
@@ -396,13 +434,13 @@ template <typename T, class BK> class DeconvEngine : public EngineBase {
         return 0;
     }
 
-    void get_array(int id, int k, double* host) {
+    void get_array(int id, int k, const ImageRef& out) {
         if (id == ARR_NORMALIZATION) ensure_norm();
         bk.cast_out(stage64, array(id, k), npix);
-        bk.download(host, stage64, sizeof(double) * npix);
+        stage_out(bk, out, stage64, npix);
     }
-    void set_array(int id, int k, const double* host) {
-        bk.upload(stage64, host, sizeof(double) * npix);
+    void set_array(int id, int k, const ImageRef& in) {
+        stage_in(bk, stage64, in, npix);
         bk.cast_in(array(id, k), stage64, npix, 1.0);
         if (id == ARR_ESTIMATE) { have_estimate = true; invalidate_estimate_spectrum(); }
         if (id == ARR_NORMALIZATION) have_norm = true;
@@ -469,25 +507,25 @@ template <typename T, class BK> class DeconvEngine : public EngineBase {
         return true;
     }
 
-    // Host-array forms of H / H_t for the Python methods.
-    void H_host(const double* x, double* out) {
-        bk.upload(stage64, x, sizeof(double) * npix);
+    // H / H_t of the Python methods, on host arrays or caller device buffers.
+    void H(const ImageRef& x, const ImageRef& out) {
+        stage_in(bk, stage64, x, npix);
         bk.cast_in(scratch, stage64, npix, 1.0);
         T* tmp = tmp_images();
         op_H(scratch, tmp, 0, 0);
         bk.cast_out(stage64, tmp, npix * K);
-        bk.download(out, stage64, sizeof(double) * npix * K);
+        stage_out(bk, out, stage64, npix * K);
         invalidate_estimate_spectrum();
     }
-    void Ht_host(const double* y, double* out, bool normalize) {
+    void Ht(const ImageRef& y, const ImageRef& out, bool normalize) {
         T* tmp = tmp_images();
         if (normalize) ensure_norm();
-        bk.upload(stage64, y, sizeof(double) * npix * K);
+        stage_in(bk, stage64, y, npix * K);
         bk.cast_in(tmp, stage64, npix * K, 1.0);
         op_Ht_raw(tmp, scratch);
         if (normalize) bk.divide(scratch, norm, npix);
         bk.cast_out(stage64, scratch, npix);
-        bk.download(out, stage64, sizeof(double) * npix);
+        stage_out(bk, out, stage64, npix);
         invalidate_estimate_spectrum();
     }
 

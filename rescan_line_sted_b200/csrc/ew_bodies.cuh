@@ -5,7 +5,8 @@
 
 namespace lsted {
 
-enum EwOp { EW_CAST_IN = 0, EW_CAST_OUT = 1, EW_FILL = 2, EW_DIVIDE = 3, EW_RL_UPDATE = 4, EW_SUB = 5 };
+enum EwOp { EW_CAST_IN = 0, EW_CAST_OUT = 1, EW_FILL = 2, EW_DIVIDE = 3, EW_RL_UPDATE = 4, EW_SUB = 5,
+            EW_TO_STAGE = 6, EW_FROM_STAGE = 7 };
 
 template <typename T> struct EwArgs {
     T* t0;            // destination (or in/out)
@@ -14,8 +15,44 @@ template <typename T> struct EwArgs {
     double* d0;
     const double* d1;
     double s;
-    size_t n;
+    size_t n;         // items
+    size_t elems;     // EW_TO_STAGE / EW_FROM_STAGE: elements
+    int vec;          // EW_TO_STAGE / EW_FROM_STAGE: the caller buffer is 16-byte aligned
 };
+
+// Conversion between a caller's device buffer of T = float or double (the _dev entry points of
+// lsted.h) and the engine's fp64 staging array.  EW_TO_STAGE: d0 = (double)t1, exact;
+// EW_FROM_STAGE: t0 = (T)d1, rounded to nearest once -- the values the host entry points
+// exchange, so a device call gives the bits of its host twin fed the same values.  With `vec`
+// item i covers the G = 16 / sizeof(T) elements from G * i with one 16-byte access of the caller
+// buffer; otherwise (a view at a storage offset is only element-aligned) item i is element i.
+template <typename T> struct alignas(16) Vec16 { T v[16 / sizeof(T)]; };
+
+template <typename T> LSTED_HD size_t stage_items(size_t elems, bool vec) {
+    const size_t G = 16 / sizeof(T);
+    return vec ? (elems + G - 1) / G : elems;
+}
+
+template <int OP, typename T> LSTED_HD void stage_apply(const EwArgs<T>& a, size_t i) {
+    const int G = (int)(16 / sizeof(T));
+    if (a.vec && (i + 1) * G <= a.elems) {
+        if (OP == EW_TO_STAGE) {
+            const Vec16<T> w = reinterpret_cast<const Vec16<T>*>(a.t1)[i];
+            for (int g = 0; g < G; ++g) a.d0[i * G + g] = (double)w.v[g];
+        } else {
+            Vec16<T> w;
+            for (int g = 0; g < G; ++g) w.v[g] = (T)a.d1[i * G + g];
+            reinterpret_cast<Vec16<T>*>(a.t0)[i] = w;
+        }
+        return;
+    }
+    const size_t e0 = a.vec ? i * G : i;
+    const size_t e1 = a.vec ? (e0 + G < a.elems ? e0 + G : a.elems) : e0 + 1;
+    for (size_t e = e0; e < e1; ++e) {
+        if (OP == EW_TO_STAGE) a.d0[e] = (double)a.t1[e];
+        else a.t0[e] = (T)a.d1[e];
+    }
+}
 
 template <int OP, typename T> LSTED_HD void ew_apply(const EwArgs<T>& a, size_t i) {
     if (OP == EW_CAST_IN) a.t0[i] = (T)(a.d1[i] * a.s);
@@ -24,6 +61,7 @@ template <int OP, typename T> LSTED_HD void ew_apply(const EwArgs<T>& a, size_t 
     else if (OP == EW_DIVIDE) a.t0[i] = a.t0[i] / a.t1[i];
     else if (OP == EW_RL_UPDATE) a.t0[i] = a.t0[i] * (a.t1[i] / a.t2[i]);  // est *= H_t(ratio)/norm
     else if (OP == EW_SUB) a.t0[i] = a.t1[i] - a.t2[i];
+    else if (OP == EW_TO_STAGE || OP == EW_FROM_STAGE) stage_apply<OP, T>(a, i);
 }
 
 

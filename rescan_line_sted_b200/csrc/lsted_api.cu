@@ -29,6 +29,10 @@ struct ApiError { int code; std::string msg; };
 
 static thread_local std::string g_error;
 static int set_error(int code, const std::string& msg) { g_error = msg; return code; }
+static lsted::ApiError arg_error(const std::string& msg) {
+    lsted::ApiError e; e.code = LSTED_ERR_ARG; e.msg = msg;
+    return e;
+}
 
 #define CUDA_CHECK(expr)                                                                  \
     do {                                                                                  \
@@ -368,6 +372,8 @@ class CudaBackend : public lsted::KernelSelection {
         CUDA_CHECK(cudaStreamCreateWithFlags(&stream_, cudaStreamNonBlocking));
         CUDA_CHECK(cudaEventCreate(&t0_));
         CUDA_CHECK(cudaEventCreate(&t1_));
+        CUDA_CHECK(cudaEventCreateWithFlags(&join_in_, cudaEventDisableTiming));
+        CUDA_CHECK(cudaEventCreateWithFlags(&join_out_, cudaEventDisableTiming));
         CUDA_CHECK(cudaDeviceGetAttribute(&num_sms_, cudaDevAttrMultiProcessorCount, device));
         ++g_live_backends;
         memset(prof_ms_, 0, sizeof(prof_ms_));
@@ -384,6 +390,8 @@ class CudaBackend : public lsted::KernelSelection {
         for (size_t i = 0; i < ev_pool_.size(); ++i) cudaEventDestroy(ev_pool_[i]);
         if (t0_) cudaEventDestroy(t0_);
         if (t1_) cudaEventDestroy(t1_);
+        if (join_in_) cudaEventDestroy(join_in_);
+        if (join_out_) cudaEventDestroy(join_out_);
         if (stream_) cudaStreamDestroy(stream_);
     }
     void activate() { CUDA_CHECK(cudaSetDevice(device_)); }
@@ -860,6 +868,51 @@ class CudaBackend : public lsted::KernelSelection {
         ew_kernel<OP, T><<<(int)blocks, kEwThreads, 0, stream_>>>(a);
         after();
     }
+    // ---- caller device buffers (the _dev entry points of lsted.h) ----
+    // `bytes` from p on must be device (or managed) memory of this handle's device, inside one
+    // allocation: checked before anything is enqueued, so no kernel sees a bad pointer
+    void check_device_buffer(const void* p, size_t bytes, const std::string& what) {
+        cudaPointerAttributes at;
+        const cudaError_t err = cudaPointerGetAttributes(&at, p);
+        if (err != cudaSuccess) {
+            cudaGetLastError();
+            throw arg_error(what + ": not a CUDA pointer (" + cudaGetErrorString(err) + ")");
+        }
+        if (at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged)
+            throw arg_error(what + ": host memory; the _dev entry points take device memory");
+        if (at.device != device_)
+            throw arg_error(what + ": memory of CUDA device " + std::to_string(at.device) +
+                            ", the handle is on device " + std::to_string(device_));
+        typedef CUresult (*range_fn)(CUdeviceptr*, size_t*, CUdeviceptr);
+        static const range_fn range = drv<range_fn>("cuMemGetAddressRange");
+        CUdeviceptr base = 0;
+        size_t size = 0;
+        if (range(&base, &size, (CUdeviceptr)p) != CUDA_SUCCESS)
+            throw arg_error(what + ": no device allocation contains this address");
+        const size_t offset = (size_t)((CUdeviceptr)p - base);
+        if (bytes > size - offset)
+            throw arg_error(what + ": the call accesses " + std::to_string(bytes) + " bytes from offset " +
+                            std::to_string(offset) + " of an allocation of " + std::to_string(size) + " bytes");
+    }
+    void check_stream(void* s) {
+        cudaStreamCaptureStatus st = cudaStreamCaptureStatusNone;
+        CUDA_CHECK(cudaStreamIsCapturing((cudaStream_t)s, &st));
+        if (st != cudaStreamCaptureStatusNone) {
+            lsted::ApiError e; e.code = LSTED_ERR_STATE;
+            e.msg = "the stream is being captured into a CUDA graph; the handle's work runs on a stream of its own";
+            throw e;
+        }
+    }
+    // the handle's stream waits for everything already enqueued on `s` ...
+    void join_in(void* s) {
+        CUDA_CHECK(cudaEventRecord(join_in_, (cudaStream_t)s));
+        CUDA_CHECK(cudaStreamWaitEvent(stream_, join_in_, 0));
+    }
+    // ... and `s` waits for the call's reads and writes
+    void join_out(void* s) {
+        CUDA_CHECK(cudaEventRecord(join_out_, stream_));
+        CUDA_CHECK(cudaStreamWaitEvent((cudaStream_t)s, join_out_, 0));
+    }
     // record_iteration's error spectrum on sides without a Stockham plan (ew_bodies.cuh)
     template <int PASS, typename T> void dft_direct(const lsted::DftArgs<T>& a) {
         const size_t n = (size_t)a.Ny * a.Nx;
@@ -951,6 +1004,7 @@ class CudaBackend : public lsted::KernelSelection {
     int prefetch_final_quarters_ = 6;   // ROW_FINAL (1024 CTAs, 592 resident): 2: 0.0271, 6: 0.0234 ms
     ncclComm_t comm_ = 0;
     cudaEvent_t t0_, t1_;
+    cudaEvent_t join_in_ = 0, join_out_ = 0;   // stream order with the caller's stream (_dev calls)
     int num_sms_;
     std::vector<cudaEvent_t> ev_pool_;
     struct Span { int kind; size_t e0, e1; };
@@ -996,6 +1050,8 @@ class CudaBackend : public lsted::KernelSelection {
 
 #define LSTED_BACKEND CudaBackend
 #include "api_deconv.inl"
+static_assert(has_caller_streams<CudaBackend>::value,
+              "the _dev entry points check buffers and join streams on the GPU");
 
 // ---------------------------------------------------------------------------
 // Core entry points

@@ -75,7 +75,7 @@ template <typename T, class BK> class TiledEngine : public EngineBase {
     ~TiledEngine() {
         void* all[] = {true_object, estimate, norm, noiseless, noisy, ratio, win1, win2, winK,
                        stage64, object64, partial, halo_send, halo_recv, stage_region,
-                       ft_scratch, tw_dx, tw_dy, spec_direct};
+                       tmp1, tw_dx, tw_dy, spec_direct};
         for (size_t i = 0; i < sizeof(all) / sizeof(all[0]); ++i) bk.free(all[i]);
     }
 
@@ -163,7 +163,7 @@ template <typename T, class BK> class TiledEngine : public EngineBase {
     // image there (the caller passes the gathered estimate instead).
     bool ft_error(const double* image_host, double* out_host) {
         if (!image_host && world > 1) return false;
-        if (!ft_scratch) {
+        if (!spec_direct) {
             std::vector<cplx<double> > tw;
             tw.resize(Nx); fill_twiddles<double>(Nx, tw.data());
             tw_dx = (cplx<double>*)bk.alloc(sizeof(cplx<double>) * Nx);
@@ -172,19 +172,19 @@ template <typename T, class BK> class TiledEngine : public EngineBase {
             tw_dy = (cplx<double>*)bk.alloc(sizeof(cplx<double>) * Ny);
             bk.upload(tw_dy, tw.data(), sizeof(cplx<double>) * Ny);
             spec_direct = (cplx<double>*)bk.alloc(sizeof(cplx<double>) * npix);
-            ft_scratch = (T*)bk.alloc(sizeof(T) * npix);
             bk.sync();
         }
+        T* diff = image_tmp();
         const T* x = estimate;
         if (image_host) {
             bk.upload(stage64, image_host, sizeof(double) * npix);
-            bk.cast_in(ft_scratch, stage64, npix, 1.0);
-            x = ft_scratch;
+            bk.cast_in(diff, stage64, npix, 1.0);
+            x = diff;
         }
-        bk.subtract(ft_scratch, x, true_object, npix);
+        bk.subtract(diff, x, true_object, npix);
         DftArgs<T> da;
         memset(&da, 0, sizeof(da));
-        da.real_in = ft_scratch; da.spec = spec_direct; da.twx = tw_dx; da.twy = tw_dy;
+        da.real_in = diff; da.spec = spec_direct; da.twx = tw_dx; da.twy = tw_dy;
         da.logmag = stage64; da.Ny = Ny; da.Nx = Nx;
         bk.template dft_direct<0, T>(da);
         bk.template dft_direct<1, T>(da);
@@ -234,7 +234,7 @@ template <typename T, class BK> class TiledEngine : public EngineBase {
     // The staged object has a buffer of its own: stage64 is the host-transfer scratch of every
     // get / set / H / H_t / ft_error, any of which may run between upload_object and simulate
     // (a frame loop uploads once and simulates a new noise field per frame).
-    void upload_object(const double* obj_host) { bk.upload(object64, obj_host, sizeof(double) * npix); }
+    void upload_object(const ImageRef& obj) { stage_in(bk, object64, obj, npix); }
     void simulate(double total_brightness, bool rescale, unsigned long long seed) {
         double s = 1.0;
         if (rescale) s = total_brightness / bk.sum(object64, npix, partial);
@@ -250,7 +250,7 @@ template <typename T, class BK> class TiledEngine : public EngineBase {
     }
     void create_data(const double* obj_host, double total_brightness, bool rescale,
                      unsigned long long seed) {
-        upload_object(obj_host);
+        upload_object(host_image(obj_host));
         simulate(total_brightness, rescale, seed);
     }
 
@@ -323,7 +323,7 @@ template <typename T, class BK> class TiledEngine : public EngineBase {
         a.src_img = bpix; a.src_pitch = E.w(); a.src_off = (size_t)(r.y0 - E.y0) * E.w() + (r.x0 - E.x0);
         bk.launch_rect(a);
     }
-    void get_array(int id, int k, double* host) {
+    void get_array(int id, int k, const ImageRef& out) {
         if (id == ARR_NORMALIZATION) ensure_norm();
         if (id == ARR_NOISELESS || id == ARR_NOISY) {
             place_region((id == ARR_NOISY ? noisy : noiseless) + bpix * k, O);
@@ -343,10 +343,10 @@ template <typename T, class BK> class TiledEngine : public EngineBase {
             bk.cast_out(stage64, id == ARR_TRUE_OBJECT ? true_object
                                  : id == ARR_ESTIMATE ? estimate : norm, npix);
         }
-        bk.download(host, stage64, sizeof(double) * npix);
+        stage_out(bk, out, stage64, npix);
     }
-    void set_array(int id, int k, const double* host) {
-        bk.upload(stage64, host, sizeof(double) * npix);
+    void set_array(int id, int k, const ImageRef& in) {
+        stage_in(bk, stage64, in, npix);
         if (id == ARR_NOISELESS || id == ARR_NOISY) {
             T* dst = (id == ARR_NOISY ? noisy : noiseless) + bpix * k;
             RectArgs<double> a;
@@ -362,33 +362,32 @@ template <typename T, class BK> class TiledEngine : public EngineBase {
         if (id == ARR_ESTIMATE) { have_estimate = true; halo_fresh = true; }
         if (id == ARR_NORMALIZATION) have_norm = true;
     }
-    // Host-array operators reuse `ratio` as the K-image temporary (it is rebuilt by
-    // every iteration anyway).
-    void H_host(const double* x, double* out) {
-        if (world > 1) throw std::string("H/H_t on host arrays need an unsharded handle");
-        T* xin = (T*)bk.alloc(sizeof(T) * npix);
-        bk.upload(stage64, x, sizeof(double) * npix);
+    // H / H_t on full-size images (host arrays or caller device buffers) reuse `ratio` as the
+    // K-image temporary (it is rebuilt by every iteration anyway).  The one-image temporary is
+    // kept rather than freed: cudaFree would wait for the whole device.
+    void H(const ImageRef& x, const ImageRef& out) {
+        if (world > 1) throw std::string("H/H_t on full-size images need an unsharded handle");
+        T* xin = image_tmp();
+        stage_in(bk, stage64, x, npix);
         bk.cast_in(xin, stage64, npix, 1.0);
         apply_H(xin, ratio);
         for (int k = 0; k < K; ++k) {
             bk.cast_out(stage64, ratio + npix * k, npix);
-            bk.download(out + npix * k, stage64, sizeof(double) * npix);
+            stage_out(bk, out.at(npix * k), stage64, npix);
         }
-        bk.free(xin);
     }
-    void Ht_host(const double* y, double* out, bool normalize) {
-        if (world > 1) throw std::string("H/H_t on host arrays need an unsharded handle");
+    void Ht(const ImageRef& y, const ImageRef& out, bool normalize) {
+        if (world > 1) throw std::string("H/H_t on full-size images need an unsharded handle");
         if (normalize) ensure_norm();
-        T* res = (T*)bk.alloc(sizeof(T) * npix);
+        T* res = image_tmp();
         for (int k = 0; k < K; ++k) {
-            bk.upload(stage64, y + npix * k, sizeof(double) * npix);
+            stage_in(bk, stage64, y.at(npix * k), npix);
             bk.cast_in(ratio + npix * k, stage64, npix, 1.0);
         }
         apply_Ht_raw(ratio, res);
         if (normalize) bk.divide(res, norm, npix);
         bk.cast_out(stage64, res, npix);
-        bk.download(out, stage64, sizeof(double) * npix);
-        bk.free(res);
+        stage_out(bk, out, stage64, npix);
     }
 
   private:
@@ -408,8 +407,12 @@ template <typename T, class BK> class TiledEngine : public EngineBase {
     T *true_object, *estimate, *norm, *noiseless, *noisy, *ratio, *win1, *win2, *winK;
     T *halo_send, *halo_recv;
     double *stage64, *object64, *partial, *stage_region;
-    T* ft_scratch = 0;                                      // ft_error (lazy)
-    cplx<double>*tw_dx = 0, *tw_dy = 0, *spec_direct = 0;
+    T* tmp1 = 0;                                            // one full-size image: ft_error, H, H_t (lazy)
+    cplx<double>*tw_dx = 0, *tw_dy = 0, *spec_direct = 0;   // ft_error (lazy)
+    T* image_tmp() {
+        if (!tmp1) tmp1 = (T*)bk.alloc(sizeof(T) * npix);
+        return tmp1;
+    }
 
     // Tile (ty, tx) of the global tile grid; `region` = the big arrays hold the rank's
     // rectangle E rather than the full image.  Only pixels of O are written back.

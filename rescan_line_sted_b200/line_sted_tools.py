@@ -631,6 +631,12 @@ class Deconvolver:
     fresh numpy array, assigning `noisy_measurement` / `estimate` uploads
     (that is the injection point for a given noise field).  Arrays handed
     out are copies: mutate-in-place does not write through, assign instead.
+
+    CUDA tensors (float32 or float64, C-contiguous, on the handle's device)
+    take a path without host copies, ordered on the current torch stream:
+    `create_data_from_object`, `H` and `H_t` accept them and return tensors,
+    the `noisy_measurement` / `estimate` setters accept them, and
+    `tensor(name)` reads an attribute as tensors.
     """
 
     def __init__(self, psfs, output_prefix=None, verbose=True):
@@ -690,6 +696,12 @@ class Deconvolver:
                 self._have.add(which)
         return self._handle
 
+    def _check_tensor(self, t, what):
+        """A (1, Ny, Nx) CUDA tensor on the handle's device (checked before any
+        handle is built or any call crosses into the library)."""
+        device = self._handle.device if self._handle is not None else _device()
+        return _lib.check_tensor(t, (1, None, None), device, what)
+
     def _need(self, what, name):
         if self._handle is None or what not in self._have:
             raise AttributeError("'Deconvolver' object has no attribute '%s'"
@@ -712,6 +724,17 @@ class Deconvolver:
 
     @noisy_measurement.setter
     def noisy_measurement(self, value):
+        value = list(value)
+        if value and _lib.is_tensor(value[0]):
+            if len(value) != len(self.psfs):
+                raise ValueError('need one measurement per PSF')
+            for v in value:
+                self._check_tensor(v, 'each measurement')
+            h = self._engine(value[0].shape)
+            for k, v in enumerate(value):
+                h.set_tensor(_lib.NOISY, k, v)
+            self._have.add(_lib.NOISY)
+            return
         value = [np.asarray(v, dtype=np.float64) for v in value]
         if len(value) != len(self.psfs):
             raise ValueError('need one measurement per PSF')
@@ -727,15 +750,47 @@ class Deconvolver:
 
     @estimate.setter
     def estimate(self, value):
-        value = np.asarray(value, dtype=np.float64)
-        h = self._engine(value.shape)
-        h.set(_lib.ESTIMATE, 0, value)
+        if _lib.is_tensor(value):
+            self._check_tensor(value, 'estimate')
+            self._engine(value.shape).set_tensor(_lib.ESTIMATE, 0, value)
+        else:
+            value = np.asarray(value, dtype=np.float64)
+            h = self._engine(value.shape)
+            h.set(_lib.ESTIMATE, 0, value)
         self._have.add(_lib.ESTIMATE)
 
     @property
     def H_t_normalization(self):
         return self._need(_lib.NORMALIZATION,
                           'H_t_normalization').get(_lib.NORMALIZATION)
+
+    _ATTRIBUTES = {'true_object': _lib.TRUE_OBJECT,
+                   'noiseless_measurement': _lib.NOISELESS,
+                   'noisy_measurement': _lib.NOISY,
+                   'estimate': _lib.ESTIMATE,
+                   'H_t_normalization': _lib.NORMALIZATION}
+
+    def tensor(self, name, dtype=None):
+        """Extension: attribute `name` as CUDA tensors of `dtype` (torch.float64 by
+        default) on the handle's device, without a host copy -- a (1, Ny, Nx)
+        tensor, or for the per-PSF measurements a list of (1, Ny, Nx) views of one
+        (K, Ny, Nx) tensor.  Ordered on the current torch stream."""
+        import torch
+        if name not in self._ATTRIBUTES:
+            raise ValueError('tensor(): name must be one of %s, got %r'
+                             % (', '.join(sorted(self._ATTRIBUTES)), name))
+        dtype = torch.float64 if dtype is None else dtype
+        if dtype not in (torch.float32, torch.float64):
+            raise TypeError('tensor(): dtype must be torch.float32 or torch.float64')
+        which = self._ATTRIBUTES[name]
+        h = self._need(which, name)
+        if which not in (_lib.NOISELESS, _lib.NOISY):
+            return h.get_tensor(which, 0, dtype)
+        out = torch.empty((h.K, h.Ny, h.Nx), dtype=dtype,
+                          device=torch.device('cuda', h.device))
+        for k in range(h.K):
+            h.get_tensor(which, k, out=out[k:k + 1])
+        return [out[k:k + 1] for k in range(h.K)]
 
     # -- the reference's methods ---------------------------------------------
     def create_data_from_object(
@@ -747,16 +802,24 @@ class Deconvolver:
         """Forward model + shot noise (ref:496-512).  The Poisson field comes
         from the in-kernel Philox generator: `random_seed` selects its
         stream; without a seed one is drawn from numpy's global generator
-        (so `np.random.seed` upstream still makes a run repeatable)."""
+        (so `np.random.seed` upstream still makes a run repeatable).
+        `obj` may be a float32 / float64 CUDA tensor of shape (1, Ny, Nx)."""
+        tensor = _lib.is_tensor(obj)
+        if tensor:
+            self._check_tensor(obj, 'obj')
         assert len(obj.shape) == 3
-        assert obj.dtype == np.float64
+        assert tensor or obj.dtype == np.float64
         h = self._engine(obj.shape)
         if random_seed is None:
             random_seed = int(np.random.randint(0, 2 ** 31 - 1)) * 2 ** 31 + \
                 int(np.random.randint(0, 2 ** 31 - 1))
         # like the reference, new data leave `estimate` and `num_iterations` alone
-        h.create_data(obj, total_brightness, int(random_seed) % 2 ** 64,
-                      reset_estimate=False)
+        if tensor:
+            h.upload_object_tensor(obj)
+            h.simulate(total_brightness, int(random_seed) % 2 ** 64, reset_estimate=False)
+        else:
+            h.create_data(obj, total_brightness, int(random_seed) % 2 ** 64,
+                          reset_estimate=False)
         self._data_version += 1
         self._have |= {_lib.TRUE_OBJECT, _lib.NOISELESS, _lib.NOISY}
         return None
@@ -839,7 +902,12 @@ class Deconvolver:
 
     def H(self, x):
         """Expected noiseless measurement operator (ref:567-577): one
-        clipped linear 'same' convolution per PSF, as a list."""
+        clipped linear 'same' convolution per PSF, as a list.  A CUDA tensor
+        gives views of one (K, Ny, Nx) tensor of its dtype."""
+        if _lib.is_tensor(x):
+            self._check_tensor(x, 'x')
+            out = self._engine(x.shape).H_tensor(x)
+            return [out[k:k + 1] for k in range(out.shape[0])]
         x = np.asarray(x, dtype=np.float64)
         h = self._engine(x.shape)
         out = h.H(x)
@@ -847,10 +915,22 @@ class Deconvolver:
 
     def H_t(self, y, normalize=True):
         """Transpose operator (ref:579-594), by default normalised so that
-        H_t(ones) == ones."""
-        y = [np.asarray(v, dtype=np.float64) for v in y]
-        h = self._engine(y[0].shape)
-        out = h.Ht(np.concatenate(y, axis=0), normalize)
+        H_t(ones) == ones.  A list of CUDA tensors gives a tensor."""
+        y = list(y)
+        if y and _lib.is_tensor(y[0]):
+            for v in y:
+                self._check_tensor(v, 'each image of y')
+            if len({(v.shape, v.dtype) for v in y}) != 1:
+                raise ValueError('the images of y must share one shape and dtype')
+            h = self._engine(y[0].shape)
+            if len(y) != h.K:
+                raise ValueError('need one image per PSF (%d), got %d' % (h.K, len(y)))
+            import torch
+            out = h.Ht_tensor(torch.cat(y, dim=0), normalize)
+        else:
+            y = [np.asarray(v, dtype=np.float64) for v in y]
+            h = self._engine(y[0].shape)
+            out = h.Ht(np.concatenate(y, axis=0), normalize)
         if normalize:
             self._have.add(_lib.NORMALIZATION)
         return out
